@@ -5,6 +5,7 @@ Contract (see DESIGN.md "Measurement"):
   python bench.py --gpus N --steps K --warmup W            -> ONE JSON line (this repo's CUDA path)
   python bench.py --impl reference --gpus N --steps K ...   -> ONE JSON line (CPU restatement of the
                                                                reference's FFT path, all host cores)
+  python bench.py ... --dump-outputs DIR                    -> also DIR/matmult_elliptic.npy, the last timed step's result
 A "step" is one MatMult_Elliptic application (elliptic.C:297-339) on the 128^3 grid with a
 variable-coefficient state (eta, deta, gradu populated by one FormFunction call, gamma=4, exponent=2),
 on N(0,1) synthetic input (numpy default_rng(0)), SURVEY.md 8(d).
@@ -570,6 +571,20 @@ def child_main(name, out=None):
     return 0
 
 
+def dump_outputs(out_dir, V, G, torch, dist, world, rank, dev):
+    """--dump-outputs DIR: what the last timed step returned to its caller, the MatMult_Elliptic result V over all interior
+    nodes of the global grid, as DIR/matmult_elliptic.npy (float64, 126^3 values, 16 MB).  The inputs are seeded, so two
+    builds run with the same arguments can be compared output for output."""
+    if world > 1:  # each rank holds its slab of V: place it in a zero global vector and sum (exact, the slabs are disjoint)
+        full = torch.zeros(G.gtotal, dtype=torch.float64, device=dev)
+        full[G.goff:G.goff + G.g] = V
+        dist.all_reduce(full)
+        V = full
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, "matmult_elliptic.npy"), V.cpu().numpy())
+
+
 def run_cuda(args):
     import torch
     import torch.distributed as dist
@@ -626,6 +641,8 @@ def run_cuda(args):
         b.record()
     barrier()
     launches = sp.launch_count() - l0
+    dump_dir = getattr(args, "dump_outputs", None)
+    V_last = V.clone() if dump_dir else None  # (the L2-warm loop below overwrites V)
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = sum(step_ms)
     # back-to-back (L2-warm) figure for context
@@ -750,6 +767,8 @@ def run_cuda(args):
         if world == 1 and not args.no_ksp:
             line["ksp"] = run_child("ksp", limit_s=240)
         print(json.dumps(line))
+    if dump_dir:
+        dump_outputs(dump_dir, V_last, G, torch, dist, world, rank, dev)
     if world > 1:
         dist.destroy_process_group()
     if not parity["ok"]:
@@ -761,7 +780,9 @@ def run_cuda(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline figure (value, ms_per_step); the context figures time max(STEPS, 2000) (value_l2_warm), "
+                         "max(STEPS, 200) (e2e) and max(STEPS // 2, 5) (stokes) steps so that each is a steady-state measurement")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="cuda", choices=["cuda", "reference"])
     ap.add_argument("--path", type=int, default=None, help="kernel path override (1 generic, 2 fused)")
@@ -769,9 +790,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the per-P sweep (ChebMult, MatMult_Elliptic on every path, device FormJacobian)")
     ap.add_argument("--no-ksp", action="store_true", help="skip the secondary 'KSP time to rtol 1e-10' measurement")
     ap.add_argument("--no-stokes", action="store_true", help="skip the StokesMatMult 128^3 object (BASELINE config 5's operator at this N, with its parity check)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step to DIR/matmult_elliptic.npy (float64) after the run")
     ap.add_argument("--child", default=None, choices=["p_sweep", "ksp", "stokes_oracle"], help=argparse.SUPPRESS)
     ap.add_argument("--out", default=None, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.child:
         return child_main(args.child, args.out)
     if args.impl == "reference":
