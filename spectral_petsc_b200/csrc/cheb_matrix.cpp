@@ -24,6 +24,8 @@ static std::vector<long double> cgl_diff_matrix_ld(int P) {
         v = (2.0L * n * n + 1.0L) / 6.0L;
       } else if (i == n) {
         v = -(2.0L * n * n + 1.0L) / 6.0L;
+      } else if (2 * i == n) {
+        v = 0.0L;  // x_i = 0 at the middle node of an odd P; cosl(pi * i / n) would leave about 1e-20 here
       } else {
         long double s = sinl(pi * (long double)i / n);
         long double c = cosl(pi * (long double)i / n);

@@ -31,6 +31,21 @@ def test_even_odd_halves_reproduce_the_differentiation_matrix(P):
     assert np.abs(y - ref).max() <= 2e-14 * np.abs(ref).max()
 
 
+def test_kernel_matrix_is_the_rounded_exact_matrix():
+    """Every entry of the double matrix the dense kernel applies is within 1.25 u of the exact CGL entry (one rounding to double of a
+    long-double value that is itself off by up to about 0.16 u next to the corners, where sinl(pi i / n) is small), which is what the
+    bound C = P + 8 of oracle.highprec.check assumes.  An exact zero stays zero: the middle diagonal entry of an odd P (x_i = 0) once
+    held about 1e-20, which the dense kernel multiplied into the middle row."""
+    from oracle import highprec
+
+    for P in range(2, 301):
+        D = sp.cheb_matrix(P)
+        ref = highprec.cgl_matrix(P)
+        assert np.all(np.abs(D - ref) <= 1.25 * 2.0 ** -53 * np.abs(ref)), P
+        if P % 2:
+            assert D[P // 2, P // 2] == 0.0
+
+
 def test_even_odd_matches_the_unpadded_halves_for_multiples_of_16():
     for P in (16, 32, 64, 128):
         D = sp.cheb_matrix(P)

@@ -25,6 +25,10 @@ def libmock(tmp_path_factory):
     ("test_zz4_gpu_optins", [], 12),
     ("test_zz3_gpu_drivers", ["test_elliptic_config1_and_nonlinear", "test_stokes_continuation_and_vtk"], 2),
     ("test_gpu_solvers", [], 5),  # green on the B200 in round 1; kept here as the regression net of the Python solver orchestration
+    # the row-wise bounds against oracle/highprec.py must also hold for the double's plain dense products: C is not too tight
+    ("test_gpu_cheb", ["test_cheb_mult_matches_oracle", "test_misaligned_views"], 204),
+    ("test_gpu_elliptic", ["test_function_and_matmult_match_oracle"], 25),
+    ("test_gpu_stokes", ["test_shells_match_oracle"], 14),
 ])
 def test_dry_run(libmock, module, filters, expect):
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "support", "dry_run_gpu_tests.py"), libmock, module] + filters,

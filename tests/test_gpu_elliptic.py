@@ -1,10 +1,12 @@
 """GPU parity of MatMult_Elliptic / FormFunction (C ABI) against the oracle restatement of
-elliptic.C on identical inputs; bar 1e-12 max-norm relative on random inputs."""
+elliptic.C on identical inputs; bar 1e-12 max-norm relative on random inputs.  Componentwise, the gradient, the MatMult and the
+residual are also checked against the long-double reference (oracle/highprec.py) with derived bounds."""
 import numpy as np
 import pytest
 import torch
 
 import spectral_petsc_b200 as sp
+from oracle import highprec as hp
 from oracle.elliptic import MatElliptic
 from conftest import rel_max
 
@@ -26,6 +28,38 @@ CASES = [([8, 6], 0.0, 2.0), ([8, 6], 4.0, 2.0), ([7, 6, 5], 4.0, 2.0), ([16, 16
          ([20, 20, 20], 4.0, 3.0), ([12] * 5, 0.0, 2.0), ([12] * 5, 4.0, 2.0), ([5, 4, 3, 6], 1.5, 2.0), ([33, 9], 4.0, 2.0),
          ([3, 3, 3], 4.0, 2.0), ([64, 64, 64], 4.0, 2.0)]
 
+# Grids added for a dispatch branch each, with the launches one MatMult makes there (elliptic.cu matmult_generic).  Fused path
+# (d <= 6, every extent <= 160): gradient batch with the pad in its loaders, flux, divergence batch with the crop-sum epilogue = 3
+# launches when the extents are equal, 2d + 1 when they are not (one even-odd launch per axis, deriv_eo_jobs), one more (the pad)
+# above 2^18 nodes.  Unfused path (d > 6 or an extent > 160): pad, d derivatives, flux, d "-=" derivatives, crop = 2d + 3.
+BRANCH = {
+    (40,): 3,                     # fused, d = 1: one job, nterms = 0, FormFunction's rhs in the epilogue
+    (6,) * 6: 3,                  # fused, d = 6 = SB200_EO_MAX_JOBS: the largest batch, 5 terms in the crop-sum epilogue
+    (7, 6, 5, 6, 7, 5): 13,       # fused, d = 6, unequal extents: one launch per axis
+    (5, 4, 6, 3, 5, 4, 3): 17,    # unfused, d = 7
+    (4,) * 9: 21,                 # unfused, d = 9, m = 2^18 exactly
+    (3, 4) * 5: 23,               # unfused, d = 10 (the largest rank)
+    (170, 12): 7,                 # unfused, axis 0 on the dense kernel (LEFT tiles, partial last tile)
+    (12, 170): 7,                 # unfused, axis 1 on the dense kernel (RIGHT tiles)
+    (161, 9, 7): 9,               # unfused, the first extent past the even-odd reach
+    (63, 64, 65): 7,              # fused, unequal extents just below 2^18 nodes (fused pad), odd / EXACT / MT-step extents
+    (64, 64, 65): 8,              # fused, unequal extents above 2^18: pad_kernel, then one launch per axis
+    (65, 65, 65): 4,              # fused, equal extents above 2^18: pad + one batch, odd P (scalar loaders, MT = 5 at P = 65)
+    (129, 129, 33): 8,            # fused, unequal extents above 2^18, MT = 9 on axes 0 / 1
+}
+CASES += [(list(dim), 4.0, 2.0) for dim in BRANCH]
+
+
+def check_matmult(G, dim, U, V):
+    """V = MatMult(U) on the device, componentwise against the long-double chain fed with the device's own eta, deta and gradu
+    (C = 2 P_max + 16 + d, oracle.highprec.elliptic_matmult).  Returns max |err| / (u M)."""
+    state = [G.get_state(k).cpu().numpy() for k in range(2 + len(dim))]
+    ref, M = hp.elliptic_matmult(dim, state[0], state[1], state[2:], U)
+    C = 2 * max(dim) + 16 + len(dim)
+    r, k = hp.check(V, ref, M, C)
+    assert r <= 1, (r, k)
+    return r * C
+
 
 @pytest.mark.parametrize("dim,gamma,exponent", CASES, ids=lambda v: str(v))
 def test_function_and_matmult_match_oracle(cuda, dim, gamma, exponent):
@@ -40,11 +74,32 @@ def test_function_and_matmult_match_oracle(cuda, dim, gamma, exponent):
     assert rel_max(G.get_state(1).cpu().numpy(), O.deta) < 1e-14 or np.abs(O.deta).max() == 0
     for k in range(O.d):
         assert rel_max(G.get_state(2 + k).cpu().numpy(), O.gradu[k]) < TOL
+    # componentwise: the gradient (C = P_k + 8) and the residual from the device's eta (C = 2 P_max + 16 + d)
+    w0, grads = hp.elliptic_gradient(dim, Us, O.dirichlet)
+    worst = {}
+    for k, (g, M) in enumerate(grads):
+        r, i = hp.check(G.get_state(2 + k).cpu().numpy(), g, M, dim[k] + 8)
+        assert r <= 1, (k, r, i)
+        worst["gradient"] = max(worst.get("gradient", 0.0), r * (dim[k] + 8))
+    C = 2 * max(dim) + 16 + len(dim)
+    Fr, MF = hp.elliptic_residual(dim, G.get_state(0).cpu().numpy(), Us, O.dirichlet, O.b)
+    r, i = hp.check(Fg.cpu().numpy(), Fr, MF, C)
+    assert r <= 1, (r, i)
+    worst["FormFunction"] = r * C
     U = rng0.standard_normal(O.g)
     Vo = O.mat_mult(U)
-    Vg = G.mat_mult(torch.from_numpy(U).to(cuda))
+    Ud = torch.from_numpy(U).to(cuda)
+    n0 = sp.launch_count()
+    Vg = G.mat_mult(Ud)
+    launches = sp.launch_count() - n0
     assert rel_max(Vg.cpu().numpy(), Vo) < TOL
+    worst["MatMult"] = check_matmult(G, dim, U, Vg.cpu().numpy())
+    print("err/(uM) elliptic %s: %s" % (dim, ", ".join("%s %.3f" % kv for kv in worst.items())))
     assert np.array_equal(G.mat_mult_host(U), Vg.cpu().numpy())
+    # the branch the grid was picked for (the CPU test double launches nothing: launch_count stays 0 there)
+    if tuple(dim) in BRANCH and launches:
+        assert launches == BRANCH[tuple(dim)], (launches, G.kernel_name())
+        assert G.kernel_name().startswith("generic path")
 
 
 def test_K3_exact2_residual(cuda):
@@ -132,6 +187,7 @@ def test_persistent_chain_at_96(cuda, dim):
     V1 = G.mat_mult(Ud).cpu().numpy()
     assert rel_max(V0, Vo) < TOL and rel_max(V1, Vo) < TOL and rel_max(V0, V1) < 1e-13
     assert np.array_equal(V0, V0b)
+    print("err/(uM) persistent chain %s: %.3f" % (dim, check_matmult(G, dim, U, V0)))
 
 
 def test_fused_path_rejects_unsupported_extents(cuda):
