@@ -48,24 +48,28 @@ __device__ __forceinline__ void eo_gemm(const double* __restrict__ Ae, const dou
                                         double (&b)[EO<P>::MT][2], int g, int t);
 
 // NT-block variant: one set of matrix fragments feeds NT line-blocks (block j at Xw + j*BE).
+// Tile range: only the TN pair tiles [i0, i0 + TN) are accumulated (acc[j][i] <-> tile i0 + i), so that two warps can split one
+// item's M dimension; every element keeps the k-loop of the whole-item product.
 // SB200_KSPLIT == 2: even and odd k-steps accumulate into two independent register sets that are added at the end - 2 x 2 x MT x NT
 // independent DMMAs between dependent ones, enough for ONE warp to keep the FP64 tensor pipe busy (the dependent-issue latency of a
 // DMMA is ~370 clk = 23 issue slots, profiles/r02_notes.md); costs 4*MT*NT more registers and changes the summation order.
 #ifndef SB200_KSPLIT
 #define SB200_KSPLIT 1
 #endif
-template <int P, int NT, bool RIGHT>
+template <int P, int NT, bool RIGHT, int TN = EO<P>::MT>
 __device__ __forceinline__ void eo_gemm_nt(const double* __restrict__ Ae, const double* __restrict__ Bo,
-                                           const double* __restrict__ Xw, double (&a)[NT][EO<P>::MT][2],
-                                           double (&b)[NT][EO<P>::MT][2], int g, int t) {
+                                           const double* __restrict__ Xw, double (&a)[NT][TN][2],
+                                           double (&b)[NT][TN][2], int g, int t, int i0 = 0) {
   using E = EO<P>;
   constexpr int BE = RIGHT ? E::BLOCK_ELEMS_RIGHT : E::BLOCK_ELEMS_LEFT;
   constexpr int KSP = (SB200_KSPLIT == 2 && E::KS % 2 == 0) ? 2 : 1;
-  double a1[KSP == 2 ? NT : 1][E::MT][2], b1[KSP == 2 ? NT : 1][E::MT][2];
+  Ae += i0 * 8 * E::LDM;
+  Bo += i0 * 8 * E::LDM;
+  double a1[KSP == 2 ? NT : 1][TN][2], b1[KSP == 2 ? NT : 1][TN][2];
 #pragma unroll
   for (int j = 0; j < NT; j++)
 #pragma unroll
-    for (int i = 0; i < E::MT; i++) {
+    for (int i = 0; i < TN; i++) {
       a[j][i][0] = a[j][i][1] = b[j][i][0] = b[j][i][1] = 0.0;
       if (KSP == 2) a1[j][i][0] = a1[j][i][1] = b1[j][i][0] = b1[j][i][1] = 0.0;
     }
@@ -80,15 +84,15 @@ __device__ __forceinline__ void eo_gemm_nt(const double* __restrict__ Ae, const 
       s[j] = p + q;
       d[j] = p - q;
     }
-    double fa[E::MT], fb[E::MT];
+    double fa[TN], fb[TN];
 #pragma unroll
-    for (int i = 0; i < E::MT; i++) {
+    for (int i = 0; i < TN; i++) {
       fa[i] = Ae[(i * 8 + g) * E::LDM + kk];
       fb[i] = Bo[(i * 8 + g) * E::LDM + kk];
     }
     const bool odd = KSP == 2 && (ks & 1);
 #pragma unroll
-    for (int i = 0; i < E::MT; i++) {
+    for (int i = 0; i < TN; i++) {
 #pragma unroll
       for (int j = 0; j < NT; j++) {
         double& a0r = odd ? a1[KSP == 2 ? j : 0][i][0] : a[j][i][0];
@@ -109,7 +113,7 @@ __device__ __forceinline__ void eo_gemm_nt(const double* __restrict__ Ae, const 
 #pragma unroll
     for (int j = 0; j < NT; j++)
 #pragma unroll
-      for (int i = 0; i < E::MT; i++) {
+      for (int i = 0; i < TN; i++) {
         a[j][i][0] += a1[j][i][0];
         a[j][i][1] += a1[j][i][1];
         b[j][i][0] += b1[j][i][0];
@@ -130,23 +134,25 @@ __device__ __forceinline__ void eo_gemm(const double* __restrict__ Ae, const dou
 //   LEFT : rows mt = i*8+g / mb = P-1-mt, lines 2t,2t+1        -> global offset base0 + m*R + 2t
 //   RIGHT: line g, rows i*8+2t,+1 / mirrors P-2-i*8-2t,+1      -> global offset (n0+g)*P + row
 // top[h]  <-> acc (a+b)[i][h];   LEFT: bot[h] <-> (b-a)[i][h];   RIGHT: bot[h] <-> (b-a)[i][1-h].
+// i counts the warp's own tiles, which start at pair row r0 (0 unless two warps split the item).
 template <int P, bool RIGHT>
 struct Own {
   long long base;  // LEFT: base0 + 2t ; RIGHT: (n0+g)*P
   long long R;
   int g, t;
+  int r0 = 0;
   __device__ __forceinline__ long long top(int i) const {
-    return RIGHT ? base + i * 8 + 2 * t : base + (long long)(i * 8 + g) * R;
+    return RIGHT ? base + r0 + i * 8 + 2 * t : base + (long long)(r0 + i * 8 + g) * R;
   }
   __device__ __forceinline__ long long bot(int i) const {
-    return RIGHT ? base + (P - 2 - i * 8 - 2 * t) : base + (long long)(P - 1 - i * 8 - g) * R;
+    return RIGHT ? base + (P - 2 - r0 - i * 8 - 2 * t) : base + (long long)(P - 1 - r0 - i * 8 - g) * R;
   }
   // shared-memory addresses of the same pairs inside the warp's block (both 16-byte aligned)
   __device__ __forceinline__ int stop(int i) const {
-    return RIGHT ? xaddr<P, true>(i * 8 + 2 * t, g) : xaddr<P, false>(i * 8 + g, 2 * t);
+    return RIGHT ? xaddr<P, true>(r0 + i * 8 + 2 * t, g) : xaddr<P, false>(r0 + i * 8 + g, 2 * t);
   }
   __device__ __forceinline__ int sbot(int i) const {
-    return RIGHT ? xaddr<P, true>(P - 2 - i * 8 - 2 * t, g) : xaddr<P, false>(P - 1 - i * 8 - g, 2 * t);
+    return RIGHT ? xaddr<P, true>(P - 2 - r0 - i * 8 - 2 * t, g) : xaddr<P, false>(P - 1 - r0 - i * 8 - g, 2 * t);
   }
 };
 
@@ -156,15 +162,16 @@ __device__ __forceinline__ void st2(double* p, double x, double y) { *reinterpre
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 
 // Warp-level L2 prefetch of the block's footprint in array x (issued long before the epilogue reads it).
-template <int P, bool RIGHT>
-__device__ __forceinline__ void prefetch_block(const double* __restrict__ x, long long base0, long long R, int lane) {
+// NPART warps that share the block each prefetch every NPART-th chunk, starting at chunk `part`.
+template <int P, bool RIGHT, int NPART = 1>
+__device__ __forceinline__ void prefetch_block(const double* __restrict__ x, long long base0, long long R, int lane, int part = 0) {
   if (RIGHT) {
     // 8 lines x P contiguous doubles starting at base0 = n0*P : 8*P*8 bytes = P/2 lines of 128 B
 #pragma unroll
-    for (int l = lane; l < P / 2; l += 32) prefetch_l2(x + base0 + l * 16);
+    for (int l = lane + 32 * part; l < P / 2; l += 32 * NPART) prefetch_l2(x + base0 + l * 16);
   } else {
 #pragma unroll
-    for (int m = lane; m < P; m += 32) prefetch_l2(x + base0 + (long long)m * R);
+    for (int m = lane + 32 * part; m < P; m += 32 * NPART) prefetch_l2(x + base0 + (long long)m * R);
   }
 }
 
@@ -226,9 +233,11 @@ __device__ __forceinline__ void load_block(double* Xw, const double* __restrict_
 // lexicographic; elliptic.C:408-409) with the homogeneous-Dirichlet pad of MatMult_Elliptic
 // (elliptic.C:305-308) applied on the fly: boundary nodes are zero-filled, so no padded copy of the
 // field is ever materialised.  All extents equal P; `axis` is the chain axis, n0 the first line.
-template <int P, bool RIGHT>
+// NPART warps that share the block each load one NPART-th of it (warp `part`: lines c with c * NPART / 8 == part on the last
+// axis, rows m with m / 4 % NPART == part otherwise).
+template <int P, bool RIGHT, int NPART = 1>
 __device__ __forceinline__ void load_block_from_U(double* Xw, const double* __restrict__ U, int d, int axis,
-                                                  unsigned n0, int lane, const SlabGeom sg) {
+                                                  unsigned n0, int lane, const SlabGeom sg, int part = 0) {
   using E = EO<P>;
   // decode the d-1 digits (base P) of line n0 over the axes other than `axis`, fastest axis first;
   // the slowest digit is whatever remains (axis 0 may have a local extent != P in slab mode)
@@ -267,8 +276,10 @@ __device__ __forceinline__ void load_block_from_U(double* Xw, const double* __re
   if (RIGHT) {
     // lanes run along the line (contiguous in U); 8 lines, ceil(P/32) passes each
     constexpr int PASSES = (P + 31) / 32;
+    static_assert(8 % NPART == 0, "each part loads whole lines");
 #pragma unroll 4
-    for (int i = 0; i < 8 * PASSES; i++) {
+    for (int ip = 0; ip < 8 * PASSES / NPART; ip++) {
+      const int i = part * (8 * PASSES / NPART) + ip;
       const int c = i / PASSES, m = lane + 32 * (i % PASSES);
       if (m >= P) continue;
       const bool ok = inter && (dig_fast + c >= 1) && (dig_fast + c <= fast_hi) && m >= 1 && m <= P - 2;
@@ -279,7 +290,7 @@ __device__ __forceinline__ void load_block_from_U(double* Xw, const double* __re
     const bool okc = inter && (dig_fast + c >= 1) && (dig_fast + c <= fast_hi);
     const double* src = U + gb + c - ist_a;  // + m * ist_a  (ist_fast == 1 for the last axis)
 #pragma unroll 4
-    for (int m = lane >> 3; m < P; m += 4) {
+    for (int m = (lane >> 3) + 4 * part; m < P; m += 4 * NPART) {
       const bool ok = okc && m >= 1 && m <= P - 2;
       cp_async8(Xw + xaddr<P, false>(m, c), ok ? src + (long long)m * ist_a : U, ok);
     }

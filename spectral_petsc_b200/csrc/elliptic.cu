@@ -446,7 +446,7 @@ int EllipticCtx::matmult(const double* U, double* V, cudaStream_t s) {
     SB_CHECK(path <= 1, SB200_ERR_SUP, "slab partition: the fused path needs equal extents P in {32,64,128}");
   } else if (path == 3 || (path == 0 && elliptic_persist_supported(*this))) {
     SB_CHECK(elliptic_persist_supported(*this), SB200_ERR_SUP, "persistent path needs equal extents P % 16 == 0 between 32 and 160");
-    last_kernel = "persist_kernel<P,NWARPS,1> phases A+B (the whole MatMult step: 2 PDL-linked launches)";
+    last_kernel = "persist_kernel<P,NWARPS,1,MW> phases A+B (the whole MatMult step: 2 PDL-linked launches; MW = 2 warps per item at P = 128)";
     return elliptic_matmult_persist(*this, U, V, s);
   }
   if (path == 2 && arena.nranks == 1) {

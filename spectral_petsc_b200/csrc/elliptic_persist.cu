@@ -52,12 +52,23 @@ __device__ __forceinline__ void tl_stamp(const PersistParams& p, int slot) {
 }
 
 
-template <int P, int NT, bool RIGHT>
+template <int P, int NT, bool RIGHT, int MW = 1>
 __device__ __forceinline__ void load_item(double* Xw, const double* __restrict__ U, int d, int axis,
-                                          long long n0, int lane, const SlabGeom sg) {
+                                          long long n0, int lane, const SlabGeom sg, int part = 0) {
   constexpr int BE = RIGHT ? EO<P>::BLOCK_ELEMS_RIGHT : EO<P>::BLOCK_ELEMS_LEFT;
 #pragma unroll
-  for (int j = 0; j < NT; j++) load_block_from_U<P, RIGHT>(Xw + j * BE, U, d, axis, (unsigned)(n0 + 8 * j), lane, sg);
+  for (int j = 0; j < NT; j++) load_block_from_U<P, RIGHT, MW>(Xw + j * BE, U, d, axis, (unsigned)(n0 + 8 * j), lane, sg, part);
+}
+
+// MW == 2: the two warps of a pair (warps 2q, 2q+1 of the CTA) share one item and meet at named barrier 1 + q
+// (barrier 0 is __syncthreads); MW == 1: the item is warp-private.
+template <int MW>
+__device__ __forceinline__ void item_sync() {
+  if (MW == 1) {
+    __syncwarp();
+  } else {
+    asm volatile("bar.sync %0, 64;" ::"r"(1 + (int)(threadIdx.x >> 6)) : "memory");
+  }
 }
 
 // Flux operands of two tiles (top and bottom pair each): eta, deta, gradu.
@@ -65,12 +76,12 @@ struct FluxBuf {
   double2 e[2][2], de[2][2], gg[2][2];
 };
 
-template <int P, bool RIGHT>
+template <int P, bool RIGHT, int TN>
 __device__ __forceinline__ void flux_load(FluxBuf& f, const Own<P, RIGHT>& own, int ib, const double* __restrict__ eta,
                                           const double* __restrict__ deta, const double* __restrict__ g0) {
 #pragma unroll
   for (int ii = 0; ii < 2; ii++) {
-    if (ib + ii >= EO<P>::MT) continue;  // (odd MT: the last pair of tiles is a single tile)
+    if (ib + ii >= TN) continue;  // (odd TN: the last pair of tiles is a single tile)
     if (eta == nullptr) {
       f.e[ii][0] = f.e[ii][1] = make_double2(1.5, 1.5);
       f.de[ii][0] = f.de[ii][1] = f.gg[ii][0] = f.gg[ii][1] = make_double2(0.25, 0.25);
@@ -87,13 +98,13 @@ __device__ __forceinline__ void flux_load(FluxBuf& f, const Own<P, RIGHT>& own, 
 }
 
 // elliptic.C:319-323 for tiles ib, ib+1:  f = eta*y + (deta*w)*g0, written over w in the block.
-template <int P, bool RIGHT>
+template <int P, bool RIGHT, int TN>
 __device__ __forceinline__ void flux_apply(const FluxBuf& f, const Own<P, RIGHT>& own, int ib, double* Xj,
-                                           const double (&a)[EO<P>::MT][2], const double (&b)[EO<P>::MT][2]) {
+                                           const double (&a)[TN][2], const double (&b)[TN][2]) {
 #pragma unroll
   for (int ii = 0; ii < 2; ii++) {
     const int i = ib + ii;
-    if (i >= EO<P>::MT) continue;
+    if (i >= TN) continue;
     const int st = own.stop(i), sb = own.sbot(i);
     const double2 wt = ld2(Xj + st), wb = ld2(Xj + sb);
     const double yt0 = a[i][0] + b[i][0], yt1 = a[i][1] + b[i][1];
@@ -119,18 +130,24 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, int c0, int
 }
 
 struct NoEarly {
-  __device__ __forceinline__ void operator()() const {}
+  __device__ __forceinline__ void operator()(int) const {}
 };
 
-// after_gemm2: called once the second GEMM has read the block for the last time (the block is free): the single-GPU kernel grabs its
-// next ticket and issues that item's load there, so the load flies during the epilogue instead of after it.
-template <int P, int NT, bool RIGHT, bool DEEP, bool PENCIL = false, bool WAITDONE = false, typename F = NoEarly>
+// refill(0) runs right before the second GEMM, refill(1) right after it, refill(2) once every warp of the item has left it (the block is
+// free): the single-GPU kernel takes its next ticket around GEMM2 and issues that item's load at refill(2), so the load flies during
+// the epilogue instead of after it.
+// MW warps share the item: warp h of them owns pair tiles [h * MT / MW, (h + 1) * MT / MW) - GEMM rows, flux and epilogue - and all
+// of them read the whole block for the B fragments.
+template <int P, int NT, bool RIGHT, bool DEEP, int MW = 1, bool PENCIL = false, bool WAITDONE = false, typename F = NoEarly>
 __device__ __forceinline__ void run_item(const PersistParams& p, int axis, long long n0, const double* Ae,
                                          const double* Bo, double* Xw, int lane, const SlabMaps* maps = nullptr, double* stage = nullptr,
-                                         F after_gemm2 = F()) {
+                                         F refill = F()) {
   using E = EO<P>;
   static_assert(!(PENCIL && RIGHT), "pencil items are strided-axis items");
+  static_assert(E::MT % MW == 0 && (MW == 1 || (NT == 1 && DEEP && !PENCIL && !WAITDONE)), "split items: single-GPU, one block");
   constexpr int BE = RIGHT ? E::BLOCK_ELEMS_RIGHT : E::BLOCK_ELEMS_LEFT;
+  constexpr int TN = E::MT / MW;  // pair tiles of this warp
+  const int h = MW == 1 ? 0 : (int)(threadIdx.x >> 5) % MW;
   const int g = lane >> 2, t = lane & 3;
   LineGeom lg;
   lg.R = PENCIL ? p.Rp : p.R[axis];
@@ -146,6 +163,7 @@ __device__ __forceinline__ void run_item(const PersistParams& p, int axis, long 
     own[j].R = lg.R;
     own[j].g = g;
     own[j].t = t;
+    own[j].r0 = h * TN * 8;
   }
   const double* __restrict__ g0 = PENCIL ? p.g0_p : p.g0[axis];
   const double* __restrict__ eta_a = PENCIL ? p.eta_p : p.eta;
@@ -157,51 +175,61 @@ __device__ __forceinline__ void run_item(const PersistParams& p, int axis, long 
 #endif
   STAMP(0);
   FluxBuf f0, f1;
-  if (DEEP) flux_load<P, RIGHT>(f0, own[0], 0, etap, deta_a, g0);
+  if (DEEP) flux_load<P, RIGHT, TN>(f0, own[0], 0, etap, deta_a, g0);
 #pragma unroll
   for (int j = 0; j < NT; j++) {
-    prefetch_block<P, RIGHT>(eta_a, base0[j], lg.R, lane);
-    prefetch_block<P, RIGHT>(deta_a, base0[j], lg.R, lane);
-    prefetch_block<P, RIGHT>(g0, base0[j], lg.R, lane);
+    prefetch_block<P, RIGHT, MW>(eta_a, base0[j], lg.R, lane, h);
+    prefetch_block<P, RIGHT, MW>(deta_a, base0[j], lg.R, lane, h);
+    prefetch_block<P, RIGHT, MW>(g0, base0[j], lg.R, lane, h);
     if (RIGHT && !PENCIL) {
       // last axis: the partial sums its epilogue adds (4 dependent batches of loads) are pulled into L2 now, a whole chain ahead
-      for (int k = 0; k < p.d - 1; k++) prefetch_block<P, true>(p.part[k], base0[j], 1, lane);
+      for (int k = 0; k < p.d - 1; k++) prefetch_block<P, true, MW>(p.part[k], base0[j], 1, lane, h);
     }
   }
   cp_async_wait<0>();
-  __syncwarp();
+  item_sync<MW>();  // (MW == 2: the other warp's half of the block has landed too)
   STAMP(1);
 
-  double a[NT][E::MT][2], b[NT][E::MT][2];
-  eo_gemm_nt<P, NT, RIGHT>(Ae, Bo, Xw, a, b, g, t);
+  double a[NT][TN][2], b[NT][TN][2];
+  eo_gemm_nt<P, NT, RIGHT, TN>(Ae, Bo, Xw, a, b, g, t, h * TN);
   __syncwarp();
   STAMP(2);
 #pragma unroll
   for (int j = 0; j < NT; j++) {
     double* Xj = Xw + j * BE;
-    if (DEEP) {
-      // software pipeline: batch k+1 is in flight while batch k is applied
-      if (j > 0) flux_load<P, RIGHT>(f0, own[j], 0, etap, deta_a, g0);
+    if (MW > 1) {
+      // the first batch has been in flight since before GEMM1; registers hold one batch only, so the next is loaded after it is applied
+      item_sync<MW>();  // the other warp's GEMM1 has read the rows overwritten below
 #pragma unroll
-      for (int ib = 0; ib < E::MT; ib += 4) {  // (MT is even: tiles ib, ib+1 always exist; ib+2, ib+3 only when MT % 4 == 0 or ib + 4 <= MT)
-        if (ib + 2 < E::MT) flux_load<P, RIGHT>(f1, own[j], ib + 2, etap, deta_a, g0);
-        flux_apply<P, RIGHT>(f0, own[j], ib, Xj, a[j], b[j]);
-        if (ib + 4 < E::MT) flux_load<P, RIGHT>(f0, own[j], ib + 4, etap, deta_a, g0);
-        if (ib + 2 < E::MT) flux_apply<P, RIGHT>(f1, own[j], ib + 2, Xj, a[j], b[j]);
+      for (int ib = 0; ib < TN; ib += 2) {
+        if (ib > 0) flux_load<P, RIGHT, TN>(f0, own[j], ib, etap, deta_a, g0);
+        flux_apply<P, RIGHT, TN>(f0, own[j], ib, Xj, a[j], b[j]);
+      }
+    } else if (DEEP) {
+      // software pipeline: batch k+1 is in flight while batch k is applied
+      if (j > 0) flux_load<P, RIGHT, TN>(f0, own[j], 0, etap, deta_a, g0);
+#pragma unroll
+      for (int ib = 0; ib < TN; ib += 4) {  // (tiles ib, ib+1 always exist; ib+2, ib+3 only when TN % 4 == 0 or ib + 4 <= TN)
+        if (ib + 2 < TN) flux_load<P, RIGHT, TN>(f1, own[j], ib + 2, etap, deta_a, g0);
+        flux_apply<P, RIGHT, TN>(f0, own[j], ib, Xj, a[j], b[j]);
+        if (ib + 4 < TN) flux_load<P, RIGHT, TN>(f0, own[j], ib + 4, etap, deta_a, g0);
+        if (ib + 2 < TN) flux_apply<P, RIGHT, TN>(f1, own[j], ib + 2, Xj, a[j], b[j]);
       }
     } else {
 #pragma unroll
-      for (int ib = 0; ib < E::MT; ib += 2) {
-        flux_load<P, RIGHT>(f0, own[j], ib, etap, deta_a, g0);
-        flux_apply<P, RIGHT>(f0, own[j], ib, Xj, a[j], b[j]);
+      for (int ib = 0; ib < TN; ib += 2) {
+        flux_load<P, RIGHT, TN>(f0, own[j], ib, etap, deta_a, g0);
+        flux_apply<P, RIGHT, TN>(f0, own[j], ib, Xj, a[j], b[j]);
       }
     }
   }
-  __syncwarp();
+  item_sync<MW>();  // (MW == 2: GEMM2 reads the rows the other warp has just written)
   STAMP(3);
-  eo_gemm_nt<P, NT, RIGHT>(Ae, Bo, Xw, a, b, g, t);
-  __syncwarp();  // block free again (the caller refills it while the epilogue drains)
-  after_gemm2();
+  refill(0);
+  eo_gemm_nt<P, NT, RIGHT, TN>(Ae, Bo, Xw, a, b, g, t, h * TN);
+  refill(1);
+  item_sync<MW>();  // block free again (the caller refills it while the epilogue drains)
+  refill(2);
   STAMP(4);
 
   if (XF(p, 2)) {
@@ -247,7 +275,7 @@ __device__ __forceinline__ void run_item(const PersistParams& p, int axis, long 
 #pragma unroll
     for (int j = 0; j < NT; j++) {
 #pragma unroll
-      for (int i = 0; i < E::MT; i++) {
+      for (int i = 0; i < TN; i++) {
         st2(part + own[j].top(i), a[j][i][0] + b[j][i][0], a[j][i][1] + b[j][i][1]);
         st2(part + own[j].bot(i), b[j][i][0] - a[j][i][0], b[j][i][1] - a[j][i][1]);
       }
@@ -295,7 +323,7 @@ __device__ __forceinline__ void run_item(const PersistParams& p, int axis, long 
       }
       const long long vrow = gid * (P - 2) - p.sg.goff - 1;  // V index of row m is vrow + m
 #pragma unroll
-      for (int ib = 0; ib < E::MT; ib += 4) {
+      for (int ib = 0; ib < TN; ib += 4) {  // (a split item at P = 128, TN = 4: one batch of loads per warp)
         double2 ot[4], ob[4];
 #pragma unroll
         for (int ii = 0; ii < 4; ii++) ot[ii] = ob[ii] = make_double2(0.0, 0.0);
@@ -307,7 +335,7 @@ __device__ __forceinline__ void run_item(const PersistParams& p, int axis, long 
             const double* __restrict__ pk = p.part[k];
 #pragma unroll
             for (int ii = 0; ii < 4; ii++) {
-              if (ib + ii >= E::MT) continue;  // (MT % 4 != 0: the last batch is short)
+              if (ib + ii >= TN) continue;  // (TN % 4 != 0: the last batch is short)
               lt[k][ii] = __ldcg(reinterpret_cast<const double2*>(pk + own[j].top(ib + ii)));
               lb[k][ii] = __ldcg(reinterpret_cast<const double2*>(pk + own[j].bot(ib + ii)));
             }
@@ -316,7 +344,7 @@ __device__ __forceinline__ void run_item(const PersistParams& p, int axis, long 
           for (int k = 0; k < 2; k++) {
 #pragma unroll
             for (int ii = 0; ii < 4; ii++) {
-              if (ib + ii >= E::MT) continue;
+              if (ib + ii >= TN) continue;
               ot[ii].x -= lt[k][ii].x;
               ot[ii].y -= lt[k][ii].y;
               ob[ii].x -= lb[k][ii].x;
@@ -329,13 +357,13 @@ __device__ __forceinline__ void run_item(const PersistParams& p, int axis, long 
             double2 lt[4], lb[4];
 #pragma unroll
             for (int ii = 0; ii < 4; ii++) {
-              if (ib + ii >= E::MT) continue;
+              if (ib + ii >= TN) continue;
               lt[ii] = __ldcg(reinterpret_cast<const double2*>(pk + own[j].top(ib + ii)));
               lb[ii] = __ldcg(reinterpret_cast<const double2*>(pk + own[j].bot(ib + ii)));
             }
 #pragma unroll
             for (int ii = 0; ii < 4; ii++) {
-              if (ib + ii >= E::MT) continue;
+              if (ib + ii >= TN) continue;
               ot[ii].x -= lt[ii].x;
               ot[ii].y -= lt[ii].y;
               ob[ii].x -= lb[ii].x;
@@ -347,10 +375,10 @@ __device__ __forceinline__ void run_item(const PersistParams& p, int axis, long 
 #pragma unroll
           for (int ii = 0; ii < 4; ii++) {
             const int i = ib + ii;
-            if (i >= E::MT) continue;
+            if (i >= TN) continue;
             const double yt0 = a[j][i][0] + b[j][i][0], yt1 = a[j][i][1] + b[j][i][1];
             const double yb0 = b[j][i][1] - a[j][i][1], yb1 = b[j][i][0] - a[j][i][0];
-            const int mt = i * 8 + 2 * t, mb = P - 2 - i * 8 - 2 * t;  // first row of each pair
+            const int mt = own[j].r0 + i * 8 + 2 * t, mb = P - 2 - own[j].r0 - i * 8 - 2 * t;  // first row of each pair
             if (mt > 0) p.V[vrow + mt] = ot[ii].x - yt0;
             p.V[vrow + mt + 1] = ot[ii].y - yt1;
             p.V[vrow + mb] = ob[ii].x - yb0;
@@ -443,15 +471,20 @@ constexpr int persist_maxreg(int nwarps, bool slab_a) {
   return nwarps > 8 ? (65536 / (nwarps * 32)) / 8 * 8 : (slab_a ? 216 : 255);
 }
 
-template <int P, int NWARPS, int NT, bool LASTPHASE, bool SLAB>
+// MW: warps per item (1, or 2 on one GPU: a pair of warps splits the item's pair tiles, see run_item).
+template <int P, int NWARPS, int NT, int MW, bool LASTPHASE, bool SLAB>
 __global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB && !LASTPHASE)) persist_kernel(PersistParams p, const __grid_constant__ SlabMaps maps) {
   using E = EO<P>;
+  static_assert(MW == 1 || (!SLAB && NWARPS % MW == 0 && NWARPS / MW <= 15), "pairs: single GPU, one named barrier each");
+  constexpr int NSLOT = NWARPS / MW;  // items in flight per CTA
   extern __shared__ __align__(128) double sm[];
+  __shared__ unsigned next_ticket[NSLOT];  // MW == 2: the pair's next ticket, taken by its first warp
   double* Ae = sm;
   double* Bo = sm + E::H * E::LDM;
   constexpr int BEMAX = E::BLOCK_ELEMS_RIGHT > E::BLOCK_ELEMS_LEFT ? E::BLOCK_ELEMS_RIGHT : E::BLOCK_ELEMS_LEFT;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  double* Xw = sm + E::MAT_ELEMS + warp * (NT * BEMAX);
+  const int slot = warp / MW, h = warp % MW;
+  double* Xw = sm + E::MAT_ELEMS + slot * (NT * BEMAX);
   // slab phase A: a staging block per warp for the pencil items' TMA stores (never touched by the loaders)
   double* stage = (SLAB && !LASTPHASE) ? sm + E::MAT_ELEMS + NWARPS * (NT * BEMAX) + warp * (P * 8) : nullptr;
   unsigned* sync = p.sync + (LASTPHASE ? 4 : 0);  // [0] ticket, [1] exited warps
@@ -471,13 +504,13 @@ __global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB && !LASTPHASE)) persist_
   // First ticket: static, strided over the CTAs first (warp w of CTA c takes w * gridDim.x + c), so that with fewer
   // items than warps (a slab rank at 4 or 8 GPUs) every SM sub-partition gets at most one busy warp instead of the
   // first CTAs taking everything.  Later tickets come from the global counter, which starts behind the static ones.
-  const unsigned nstatic = gridDim.x * NWARPS;
+  const unsigned nstatic = gridDim.x * NSLOT;
   auto grab = [&]() -> unsigned {
     unsigned tk = 0;
     if (lane == 0) tk = atomicAdd(sync, 1u) + nstatic;
     return __shfl_sync(0xffffffffu, tk, 0);
   };
-  const unsigned first_ticket = warp * gridDim.x + blockIdx.x;
+  const unsigned first_ticket = slot * gridDim.x + blockIdx.x;
   bool peers_ready = false;
   auto issue_load = [&](unsigned tk) {
     if (tk >= total) return;
@@ -506,10 +539,10 @@ __global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB && !LASTPHASE)) persist_
     const int arel = LASTPHASE ? 0 : tl / items_per_axis;
     const int axis = LASTPHASE ? p.d - 1 : p.first_axis + arel;
     const long long n0 = (long long)(tl - arel * items_per_axis) * (8 * NT);
-    load_item<P, NT, LASTPHASE>(Xw, p.U, p.d, axis, n0, lane, p.sg);
+    load_item<P, NT, LASTPHASE, MW>(Xw, p.U, p.d, axis, n0, lane, p.sg, h);
   };
 
-  constexpr bool DEEP = (NWARPS * NT <= 8);  // 255 registers available
+  constexpr bool DEEP = MW > 1 || (NWARPS * NT <= 8);  // 255 registers available, or a quarter of the item's accumulators per warp
   // De-phase the warps of each SM sub-partition (warp w runs on SMSP w % 4): identical items started
   // together stay in lockstep, which serialises the tensor phases against the memory phases.
   unsigned tk = 0;
@@ -555,9 +588,9 @@ __global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB && !LASTPHASE)) persist_
   while (tk < total) {
     if (SLAB && !LASTPHASE && tk >= nlocal + items0) {
       if (pencil_done) report_pencils();  // before this warp may block on the other ranks' DONE
-      run_item<P, NT, true, DEEP, false, true>(p, p.d - 1, (long long)(tk - nlocal - items0) * (8 * NT), Ae, Bo, Xw, lane);
+      run_item<P, NT, true, DEEP, 1, false, true>(p, p.d - 1, (long long)(tk - nlocal - items0) * (8 * NT), Ae, Bo, Xw, lane);
     } else if (SLAB && !LASTPHASE && tk >= nlocal) {
-      run_item<P, NT, false, DEEP, true>(p, 0, (long long)(tk - nlocal) * (8 * NT), Ae, Bo, Xw, lane, &maps, stage);
+      run_item<P, NT, false, DEEP, 1, true>(p, 0, (long long)(tk - nlocal) * (8 * NT), Ae, Bo, Xw, lane, &maps, stage);
       pencil_done++;
     } else {
       const unsigned tl = tk;
@@ -565,13 +598,25 @@ __global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB && !LASTPHASE)) persist_
       const int axis = LASTPHASE ? p.d - 1 : p.first_axis + arel;
       const long long n0 = (long long)(tl - arel * items_per_axis) * (8 * NT);
       if (SLAB) {
-        run_item<P, NT, LASTPHASE, DEEP, false, SLAB && LASTPHASE>(p, axis, n0, Ae, Bo, Xw, lane);
+        run_item<P, NT, LASTPHASE, DEEP, 1, false, SLAB && LASTPHASE>(p, axis, n0, Ae, Bo, Xw, lane);
       } else {
-        auto early = [&]() {
-          nxt = grab();
-          issue_load(nxt);
+        unsigned claimed = 0;
+        auto early = [&](int at) {
+          if (MW == 1) {
+            if (at == 2) {
+              nxt = grab();
+              issue_load(nxt);
+            }
+          } else if (at == 0) {
+            if (h == 0 && lane == 0) claimed = atomicAdd(sync, 1u) + nstatic;  // one ticket per pair; its latency hides behind GEMM2
+          } else if (at == 1) {
+            if (h == 0 && lane == 0) next_ticket[slot] = claimed;  // published by the pair barrier that follows
+          } else {
+            nxt = next_ticket[slot];
+            issue_load(nxt);  // both warps load their half of the block
+          }
         };
-        run_item<P, NT, LASTPHASE, DEEP, false, false>(p, axis, n0, Ae, Bo, Xw, lane, nullptr, nullptr, early);
+        run_item<P, NT, LASTPHASE, DEEP, MW>(p, axis, n0, Ae, Bo, Xw, lane, nullptr, nullptr, early);
       }
       if (merged) {
         __threadfence();  // this item's partial rows are visible device-wide before it checks in
@@ -600,9 +645,9 @@ __global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB && !LASTPHASE)) persist_
   }
 }
 
-template <int P, int NWARPS, int NT, bool LASTPHASE, bool SLAB>
+template <int P, int NWARPS, int NT, int MW, bool LASTPHASE, bool SLAB>
 int launch_phase(const PersistParams& p, size_t smem, int sms, cudaStream_t s) {
-  auto kern = persist_kernel<P, NWARPS, NT, LASTPHASE, SLAB>;
+  auto kern = persist_kernel<P, NWARPS, NT, MW, LASTPHASE, SLAB>;
   static bool attr[64] = {};  // the opt-in above 48 KB of dynamic shared memory is per device
   int cur = 0;
   cudaGetDevice(&cur);
@@ -639,16 +684,21 @@ int launch_phase(const PersistParams& p, size_t smem, int sms, cudaStream_t s) {
   return 0;
 }
 
-template <int P, int NWARPS, int NT>
+template <int P, int NWARPS, int NT, int MW = 1>
 int run_cfg(PersistParams& p, cudaStream_t s) {
   using E = EO<P>;
   constexpr int BEMAX = E::BLOCK_ELEMS_RIGHT > E::BLOCK_ELEMS_LEFT ? E::BLOCK_ELEMS_RIGHT : E::BLOCK_ELEMS_LEFT;
-  const size_t smem = (size_t)(E::MAT_ELEMS + NWARPS * NT * BEMAX) * sizeof(double);
-  const size_t smem_slab_a = smem + (size_t)NWARPS * P * 8 * sizeof(double);  // + the pencil items' staging blocks
+  const size_t smem = (size_t)(E::MAT_ELEMS + NWARPS / MW * NT * BEMAX) * sizeof(double);
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  if (p.nranks > 1) {
+  // start stagger per group of 4 warps (clk): split items 3000 (0 / 3000 / 6000: 0.107 / 0.089 / 0.093 ms at 128^3, profiles/r03_notes.md),
+  // whole items 6000 (profiles/r02_notes.md)
+  if (p.stagger < 0) p.stagger = MW > 1 ? 3000 : 6000;
+  if constexpr (MW > 1) {
+    SB_CHECK(p.nranks == 1, SB200_ERR_SUP, "persistent path: split items are a single-GPU configuration");
+  } else if (p.nranks > 1) {
+    const size_t smem_slab_a = smem + (size_t)NWARPS * P * 8 * sizeof(double);  // + the pencil items' staging blocks
     if (!XF(p, 32)) {
       int blocks = sms;
       if (const char* mc = getenv("SB200_MAX_CTAS")) blocks = atoi(mc) > 0 ? atoi(mc) : blocks;
@@ -667,12 +717,12 @@ int run_cfg(PersistParams& p, cudaStream_t s) {
     }
     p.nlocal_items = (unsigned)(p.nlines / (8 * NT) * (p.d - 1 - p.first_axis));
     if (NT != 1) p.bulk = 0;
-    SB_TRY((launch_phase<P, NWARPS, NT, false, true>(p, smem_slab_a, sms, s)));
-    if (!p.merged) SB_TRY((launch_phase<P, NWARPS, NT, true, true>(p, smem, sms, s)));
+    SB_TRY((launch_phase<P, NWARPS, NT, 1, false, true>(p, smem_slab_a, sms, s)));
+    if (!p.merged) SB_TRY((launch_phase<P, NWARPS, NT, 1, true, true>(p, smem, sms, s)));
     return 0;
   }
-  SB_TRY((launch_phase<P, NWARPS, NT, false, false>(p, smem, sms, s)));
-  SB_TRY((launch_phase<P, NWARPS, NT, true, false>(p, smem, sms, s)));
+  SB_TRY((launch_phase<P, NWARPS, NT, MW, false, false>(p, smem, sms, s)));
+  SB_TRY((launch_phase<P, NWARPS, NT, MW, true, false>(p, smem, sms, s)));
   return 0;
 }
 
@@ -688,15 +738,14 @@ bool elliptic_persist_supported(const EllipticCtx& e) {
 }
 
 int persist_run(int P, PersistParams& p, cudaStream_t s) {
-  static int cfg = -1, stg = -1;
-  if (cfg < 0) {
-    const char* c = getenv("SB200_PERSIST_CFG");
-    cfg = c ? atoi(c) : -1;  // default: 12 warps x 168 registers on one GPU (0.0993 ms against 0.1014 ms for 8 x 255, profiles/r02_notes.md),
-                             // 8 x 255 on a slab partition (its staging blocks need the shared memory of the extra warps' blocks)
+  static bool read_env = false;
+  static int stg = -1;
+  if (!read_env) {
     const char* g = getenv("SB200_STAGGER");
-    stg = g ? atoi(g) : 6000;
+    stg = g ? atoi(g) : -1;
+    read_env = true;
   }
-  p.stagger = stg;
+  p.stagger = stg;  // (< 0: the configuration's default, run_cfg)
 #ifdef SB200_ABLATE
   const char* xf = getenv("SB200_XFLAGS");
   p.xflags = xf ? atoi(xf) : 0;
@@ -715,14 +764,11 @@ int persist_run(int P, PersistParams& p, cudaStream_t s) {
     case 144: SB_CHECK(p.nranks == 1, SB200_ERR_SUP, "persistent path: this extent is a single-GPU instantiation"); return run_cfg<144, 8, 1>(p, s);
     case 160: SB_CHECK(p.nranks == 1, SB200_ERR_SUP, "persistent path: this extent is a single-GPU instantiation"); return run_cfg<160, 8, 1>(p, s);
     case 128:
-      switch (cfg >= 0 ? cfg : (p.nranks > 1 ? 2 : 1)) {
-        case 0: return run_cfg<128, 16, 1>(p, s);
-        case 1:
-          if (p.nranks > 1) return run_cfg<128, 8, 1>(p, s);  // (12 warps + staging blocks exceed the shared memory of an SM)
-          return run_cfg<128, 12, 1>(p, s);
-        case 3: return run_cfg<128, 8, 2>(p, s);
-        default: return run_cfg<128, 8, 1>(p, s);
-      }
+      // one GPU: 8 pairs of warps x 128 registers, each pair splitting one item (0.089 ms against 0.099 ms for 12 whole-item warps x 168
+      // registers on a B200 at 1000 W, profiles/r03_notes.md; split items at P = 64 / 96 measured slower, at 32 equal); a slab partition
+      // keeps 8 whole-item warps x 255 (its staging blocks need the shared memory of further warps' blocks)
+      if (p.nranks > 1) return run_cfg<128, 8, 1>(p, s);
+      return run_cfg<128, 16, 1, 2>(p, s);
   }
   set_last_error("persistent path: unsupported extent");
   return SB200_ERR_SUP;
