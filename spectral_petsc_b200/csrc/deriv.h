@@ -13,24 +13,9 @@ enum DerivMode { DERIV_STORE = 0, DERIV_SUB = 1, DERIV_ADD = 2 };
 // Likewise the fused crop-sum epilogue (its term loads are dependent L2 round trips of the finishing job's warps): 180 us against
 // 100 + 55 us at 128^3 for the Stokes viscous tail; small grids gain the launch
 #define SB200_FUSE_CROP_MAX_NODES (1ll << 18)
-// Forward all-to-all of the slab partition folded into the kernel that PRODUCES the operand of an axis-0 derivative: element e of the
-// local field (planes x R elements, unit stride) also goes to the pencil of the rank that owns its column - Xp_q[(i0 + ml)*Rp + (c - q*Rp)]
-// with ml = e / R, c = e % R, q = c / Rp - so no separate push kernel reads the field again.
 #ifndef SB200_MAX_RANKS
 #define SB200_MAX_RANKS 8
 #endif
-struct SlabPush {
-  double* dst[SB200_MAX_RANKS] = {};
-  int on = 0, i0 = 0;
-  long long R = 1, Rp = 1;
-#ifdef __CUDACC__
-  __device__ __forceinline__ void store(long long e, double v) const {
-    const long long ml = e / R, c = e - ml * R;
-    const int q = (int)(c / Rp);
-    dst[q][(i0 + ml) * Rp + (c - (long long)q * Rp)] = v;
-  }
-#endif
-};
 
 // Grid geometry behind the lines of a job of the even-odd kernel (only needed by its fused pad / crop modes).
 struct EoLineMap {
@@ -105,9 +90,5 @@ struct SymmArena;
 // Transpose-based derivative along the partitioned axis of a slab-distributed field (slab_deriv.cu).
 bool slab_deriv0_pencil_supported(const SymmArena& a, const DerivParams& p);
 int slab_deriv0_pencil(SymmArena& a, const DerivParams& p, int nloc, int i0, double* Xp, double* Yp, cudaStream_t s);
-int slab_deriv0_pencil_begin(SymmArena& a, const DerivParams& p, int nloc, int i0, double* Xp, cudaStream_t s);
-int slab_deriv0_pencil_finish(SymmArena& a, const DerivParams& p, int nloc, double* Xp, double* Yp, cudaStream_t s);
-// The push descriptor a producer kernel needs to fill the pencils of an axis-0 derivative of the field it writes (R elements per plane).
-SlabPush slab_make_push(const SymmArena& a, double* Xp, int i0, long long R);
 
 }  // namespace sb200

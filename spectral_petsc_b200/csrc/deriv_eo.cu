@@ -10,8 +10,6 @@
 // middle node of an odd P is folded into the matrices on the host, cheb_matrix.cpp), every warp owns an 8-line block, pulls tickets
 // from a global counter and runs  load -> even-odd DMMA GEMM -> epilogue  with no CTA barrier after the matrix load.  Executed
 // flops are half of the dense product that deriv_generic.cu performs.
-#include <cstdlib>
-
 #include "../../include/spectral_b200.h"
 #include "chain.cuh"
 #include "deriv.h"
@@ -553,16 +551,7 @@ int deriv_eo_batch(const DerivParams* jobs, int n, unsigned* sync, cudaStream_t 
     case 5: return launch_mt<5, 16>(q, s);
     case 6: return launch_mt<6, 16>(q, s);
     case 7: return launch_mt<7, 16>(q, s);
-    case 8: {
-      static int nw = -1;
-      if (nw < 0) {
-        const char* c = getenv("SB200_EO_WARPS");  // tuning hook for the P = 113..128 instantiation: 8, 12 or 16 warps per CTA
-        nw = c ? atoi(c) : 16;
-      }
-      if (nw == 8) return launch_mt<8, 8>(q, s);
-      if (nw == 12) return launch_mt<8, 12>(q, s);
-      return launch_mt<8, 16>(q, s);
-    }
+    case 8: return launch_mt<8, 16>(q, s);
     case 9: return launch_mt<9, 12>(q, s);
     case 10: return launch_mt<10, 10>(q, s);
   }

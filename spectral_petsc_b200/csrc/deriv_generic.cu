@@ -12,8 +12,6 @@
 // (elliptic.C:331-334, stokes.C:590,671) without an extra pass.
 #include "deriv.h"
 
-#include <cstdlib>
-
 #include "common.cuh"
 #include "../../include/spectral_b200.h"
 
@@ -227,14 +225,7 @@ int launch_by_P(const DerivParams& p, cudaStream_t stream) {
 int deriv_apply(const DerivParams& p, cudaStream_t stream) {
   SB_CHECK(p.P >= 2 && p.O >= 1 && p.R >= 1, SB200_ERR_USER, "deriv: bad extents");
   SB_CHECK(p.x != p.y, SB200_ERR_ARG, "deriv: x and y must not alias (chebyshev.c:127)");
-  if (p.sync && deriv_eo_supported(p)) {
-    static int use_eo = -1;
-    if (use_eo < 0) {
-      const char* c = getenv("SB200_NO_EO");
-      use_eo = (c && atoi(c)) ? 0 : 1;
-    }
-    if (use_eo) return deriv_eo_apply(p, p.sync, stream);
-  }
+  if (p.sync && deriv_eo_supported(p)) return deriv_eo_apply(p, p.sync, stream);
   if (p.npeer > 1) {
     SB_CHECK(p.O == 1 && p.nloc >= 1 && p.nloc * p.npeer == p.P, SB200_ERR_USER, "deriv: bad slab partition");
     return launch_by_P<true>(p, stream);

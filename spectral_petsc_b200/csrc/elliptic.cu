@@ -9,7 +9,6 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdlib>
 #include <vector>
 
 #include "../../include/spectral_b200.h"
@@ -312,13 +311,7 @@ EllipticCtx::~EllipticCtx() {
 // Single GPU, rank <= SB200_EO_MAX_JOBS, every extent within the even-odd kernel's reach: the generic path runs as
 // [gradient batch with the pad in its loader] -> flux -> [divergence batch with the "-=" chain and the crop in its epilogue].
 bool EllipticCtx::fusable() const {
-  static int use = -1;
-  if (use < 0) {
-    const char* c = getenv("SB200_NO_EO");
-    const char* f = getenv("SB200_NO_FUSE");
-    use = ((c && atoi(c)) || (f && atoi(f))) ? 0 : 1;
-  }
-  if (!use || arena.nranks > 1 || gd.d > SB200_EO_MAX_JOBS) return false;
+  if (arena.nranks > 1 || gd.d > SB200_EO_MAX_JOBS) return false;
   for (int k = 0; k < gd.d; k++)
     if (!deriv_eo_supported(job(k, w[0], w[1], nullptr, DERIV_STORE))) return false;
   return true;

@@ -11,8 +11,6 @@
 #include "deriv.h"
 #include "elliptic.h"
 
-#include <cstdlib>
-
 namespace sb200 {
 
 namespace {
@@ -184,7 +182,6 @@ int launch_chain(const ChainParams& p, cudaStream_t s) {
   // one persistent CTA per SM; fewer when there is not a block per warp to hand out
   long long grid = (nblocks + NWARPS - 1) / NWARPS;
   if (grid > sms) grid = sms;
-  if (const char* gs = getenv("SB200_CHAIN_GRID")) grid = atoi(gs);  // experiment knob
   if (grid < 1) grid = 1;
   kern<<<(unsigned)grid, NWARPS * 32, smem, s>>>(p);
   count_launch();

@@ -123,7 +123,8 @@ __device__ __forceinline__ void flux_apply(const FluxBuf& f, const Own<P, RIGHT>
 // DEEP: keep one flux batch in flight across GEMM1 and double-buffer the batches (needs registers).
 // PENCIL (slab mode, axis 0): n0 is the line index inside this rank's pencil; the flux operands come
 // from the pencil-layout state and the result rows are pushed to the part[0] array of the planes' owners.
-// WAITDONE (slab mode, last axis): part[0] is complete once every rank has raised its DONE flag.
+// WAITDONE (slab mode, last axis, same launch as the local axes): their partials are complete once every local item has checked in,
+// part[0] once every rank has raised its DONE flag.
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, int c0, int c1, const void* smem_src) {
   const unsigned s = (unsigned)__cvta_generic_to_shared(smem_src);
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%1, %2}], [%3];" ::"l"(map), "r"(c0), "r"(c1), "r"(s) : "memory");
@@ -284,8 +285,7 @@ __device__ __forceinline__ void run_item(const PersistParams& p, int axis, long 
     // last axis: phase A (all partials) must be complete and visible, then
     // V = crop(((0 - p_0) - p_1 ...) - D f)
     asm volatile("griddepcontrol.wait;" ::: "memory");
-    if (WAITDONE && p.merged) {
-      // same launch as the local axes: their partials are complete once every local item has checked in
+    if (WAITDONE) {
       if (lane == 0) {
         const long long t0 = clock64();
         while (*reinterpret_cast<volatile unsigned*>(p.sync + 6) < p.nlocal_items) {
@@ -465,16 +465,18 @@ __global__ void __launch_bounds__(128, 6) stage_kernel(PersistParams p) {
   }
 }
 
-// Register budget: one CTA per SM.  The slab phase-A / merged kernel keeps ~9.7K registers of the SM free so that
+// Register budget: one CTA per SM.  The slab kernel keeps ~9.7K registers of the SM free so that
 // the blocks of the stage kernel (128 threads x 76 registers) can share the SM with it (PDL overlap).
-constexpr int persist_maxreg(int nwarps, bool slab_a) {
-  return nwarps > 8 ? (65536 / (nwarps * 32)) / 8 * 8 : (slab_a ? 216 : 255);
+constexpr int persist_maxreg(int nwarps, bool slab) {
+  return nwarps > 8 ? (65536 / (nwarps * 32)) / 8 * 8 : (slab ? 216 : 255);
 }
 
 // MW: warps per item (1, or 2 on one GPU: a pair of warps splits the item's pair tiles, see run_item).
+// SLAB: one launch for every axis of a slab rank - the local axes, the axis-0 pencil items, then the last axis (LASTPHASE is false).
 template <int P, int NWARPS, int NT, int MW, bool LASTPHASE, bool SLAB>
-__global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB && !LASTPHASE)) persist_kernel(PersistParams p, const __grid_constant__ SlabMaps maps) {
+__global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB)) persist_kernel(PersistParams p, const __grid_constant__ SlabMaps maps) {
   using E = EO<P>;
+  static_assert(!(SLAB && LASTPHASE), "slab: the last axis runs in the same launch");
   static_assert(MW == 1 || (!SLAB && NWARPS % MW == 0 && NWARPS / MW <= 15), "pairs: single GPU, one named barrier each");
   constexpr int NSLOT = NWARPS / MW;  // items in flight per CTA
   extern __shared__ __align__(128) double sm[];
@@ -485,21 +487,20 @@ __global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB && !LASTPHASE)) persist_
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int slot = warp / MW, h = warp % MW;
   double* Xw = sm + E::MAT_ELEMS + slot * (NT * BEMAX);
-  // slab phase A: a staging block per warp for the pencil items' TMA stores (never touched by the loaders)
-  double* stage = (SLAB && !LASTPHASE) ? sm + E::MAT_ELEMS + NWARPS * (NT * BEMAX) + warp * (P * 8) : nullptr;
+  // slab: a staging block per warp for the pencil items' TMA stores (never touched by the loaders)
+  double* stage = SLAB ? sm + E::MAT_ELEMS + NWARPS * (NT * BEMAX) + warp * (P * 8) : nullptr;
   unsigned* sync = p.sync + (LASTPHASE ? 4 : 0);  // [0] ticket, [1] exited warps
 
   const unsigned items_per_axis = (unsigned)(p.nlines / (8 * NT));
-  // slab phase A: the local axes come first; the axis-0 pencil items follow once every rank's planes have
-  // arrived (tickets [nlocal, total))
-  const unsigned items0 = (SLAB && !LASTPHASE) ? (unsigned)(p.Rp / (8 * NT)) : 0u;
+  // slab: the local axes come first; the axis-0 pencil items follow once every rank's planes have arrived (tickets
+  // [nlocal, nlocal + items0)), the last-axis items come last
+  const unsigned items0 = SLAB ? (unsigned)(p.Rp / (8 * NT)) : 0u;
   const unsigned nlocal = LASTPHASE ? items_per_axis : items_per_axis * (p.d - 1 - p.first_axis);
-  const bool merged = SLAB && !LASTPHASE && p.merged;
-  const unsigned total = nlocal + items0 + (merged ? items_per_axis : 0u);  // merged: the last-axis items come last
+  const unsigned total = nlocal + items0 + (SLAB ? items_per_axis : 0u);
   if (!LASTPHASE) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
 
   load_matrices<P>(sm, p.Ae, p.Bo);
-  if (SLAB && threadIdx.x == 0) tl_stamp(p, LASTPHASE ? 5 : 0);
+  if (SLAB && threadIdx.x == 0) tl_stamp(p, 0);
 
   // First ticket: static, strided over the CTAs first (warp w of CTA c takes w * gridDim.x + c), so that with fewer
   // items than warps (a slab rank at 4 or 8 GPUs) every SM sub-partition gets at most one busy warp instead of the
@@ -514,11 +515,11 @@ __global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB && !LASTPHASE)) persist_
   bool peers_ready = false;
   auto issue_load = [&](unsigned tk) {
     if (tk >= total) return;
-    if (SLAB && !LASTPHASE && tk >= nlocal + items0) {
+    if (SLAB && tk >= nlocal + items0) {
       load_item<P, NT, true>(Xw, p.U, p.d, p.d - 1, (long long)(tk - nlocal - items0) * (8 * NT), lane, p.sg);
       return;
     }
-    if (SLAB && !LASTPHASE && tk >= nlocal) {
+    if (SLAB && tk >= nlocal) {
       if (!peers_ready && !XF(p, 4)) {
         // every rank must have pushed its planes of the padded input into this rank's pencil
         if (lane < p.nranks) spin_until(p.sf.f[p.rank] + SYMM_READY + lane, p.epoch, p.sf.f[p.rank]);
@@ -546,7 +547,7 @@ __global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB && !LASTPHASE)) persist_
   // De-phase the warps of each SM sub-partition (warp w runs on SMSP w % 4): identical items started
   // together stay in lockstep, which serialises the tensor phases against the memory phases.
   unsigned tk = 0;
-  if (SLAB && !LASTPHASE) {
+  if (SLAB) {
     // a first ticket may be a pencil item that waits for the peers: never hold the CTA barrier behind it
     cp_async_wait<0>();
     __syncthreads();
@@ -586,10 +587,10 @@ __global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB && !LASTPHASE)) persist_
   };
   unsigned nxt = 0;
   while (tk < total) {
-    if (SLAB && !LASTPHASE && tk >= nlocal + items0) {
+    if (SLAB && tk >= nlocal + items0) {
       if (pencil_done) report_pencils();  // before this warp may block on the other ranks' DONE
       run_item<P, NT, true, DEEP, 1, false, true>(p, p.d - 1, (long long)(tk - nlocal - items0) * (8 * NT), Ae, Bo, Xw, lane);
-    } else if (SLAB && !LASTPHASE && tk >= nlocal) {
+    } else if (SLAB && tk >= nlocal) {
       run_item<P, NT, false, DEEP, 1, true>(p, 0, (long long)(tk - nlocal) * (8 * NT), Ae, Bo, Xw, lane, &maps, stage);
       pencil_done++;
     } else {
@@ -598,7 +599,7 @@ __global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB && !LASTPHASE)) persist_
       const int axis = LASTPHASE ? p.d - 1 : p.first_axis + arel;
       const long long n0 = (long long)(tl - arel * items_per_axis) * (8 * NT);
       if (SLAB) {
-        run_item<P, NT, LASTPHASE, DEEP, 1, false, SLAB && LASTPHASE>(p, axis, n0, Ae, Bo, Xw, lane);
+        run_item<P, NT, false, DEEP, 1>(p, axis, n0, Ae, Bo, Xw, lane);
       } else {
         unsigned claimed = 0;
         auto early = [&](int at) {
@@ -618,7 +619,7 @@ __global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB && !LASTPHASE)) persist_
         };
         run_item<P, NT, LASTPHASE, DEEP, MW>(p, axis, n0, Ae, Bo, Xw, lane, nullptr, nullptr, early);
       }
-      if (merged) {
+      if (SLAB) {
         __threadfence();  // this item's partial rows are visible device-wide before it checks in
         __syncwarp();
         if (lane == 0) atomicAdd(sync + 6, 1u);
@@ -632,17 +633,26 @@ __global__ void __maxnreg__(persist_maxreg(NWARPS, SLAB && !LASTPHASE)) persist_
     }
   }
   cp_async_wait<0>();
-  if (SLAB && !LASTPHASE && pencil_done) report_pencils();
+  if (SLAB && pencil_done) report_pencils();
   // the last warp to leave re-arms the counters for the next launch
   if (lane == 0) {
     const unsigned gone = atomicAdd(sync + 1, 1u);
     if (gone == gridDim.x * NWARPS - 1) {
       sync[0] = 0;
       sync[1] = 0;
-      if (merged) sync[6] = 0;
-      if (SLAB) tl_stamp(p, LASTPHASE ? 9 : 8);
+      if (SLAB) {
+        sync[6] = 0;
+        tl_stamp(p, 8);
+      }
     }
   }
+}
+
+// Test hook SB200_MAX_CTAS: caps the grids, so that several slab ranks emulated on ONE device are all resident at the same time.
+long long cap_ctas(long long grid) {
+  const char* mc = getenv("SB200_MAX_CTAS");
+  const int lim = mc ? atoi(mc) : 0;
+  return lim > 0 && grid > lim ? lim : grid;
 }
 
 template <int P, int NWARPS, int NT, int MW, bool LASTPHASE, bool SLAB>
@@ -656,16 +666,11 @@ int launch_phase(const PersistParams& p, size_t smem, int sms, cudaStream_t s) {
     attr[cur & 63] = true;
   }
   long long items = p.nlines / (8 * NT) * (LASTPHASE ? 1 : p.d - 1 - p.first_axis);
-  if (SLAB && !LASTPHASE) items += p.Rp / (8 * NT) + (p.merged ? p.nlines / (8 * NT) : 0);
+  if (SLAB) items += p.Rp / (8 * NT) + p.nlines / (8 * NT);
   if (items <= 0) return 0;
   // one persistent CTA per SM; with fewer items than warps spread them over all SMs (a warp alone on its
   // SM sub-partition issues DMMAs ~1.5x faster than two sharing it)
-  long long grid = items < sms ? items : sms;
-  if (const char* mc = getenv("SB200_MAX_CTAS")) {
-    // test hook: several slab ranks emulated on ONE device must all be resident at the same time
-    const int lim = atoi(mc);
-    if (lim > 0 && grid > lim) grid = lim;
-  }
+  long long grid = cap_ctas(items < sms ? items : sms);
   if (grid < 1) grid = 1;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)grid);
@@ -676,7 +681,7 @@ int launch_phase(const PersistParams& p, size_t smem, int sms, cudaStream_t s) {
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
-  // phase B may start while phase A drains; slab phase A may start while the stage kernel pushes
+  // phase B may start while phase A drains; the slab kernel may start while the stage kernel pushes
   cfg.numAttrs = (LASTPHASE || SLAB) ? 1 : 0;
   static const SlabMaps no_maps = {};
   SB_CUDA(cudaLaunchKernelEx(&cfg, kern, p, (SLAB && p.maps) ? *p.maps : no_maps));
@@ -694,14 +699,13 @@ int run_cfg(PersistParams& p, cudaStream_t s) {
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   // start stagger per group of 4 warps (clk): split items 3000 (0 / 3000 / 6000: 0.107 / 0.089 / 0.093 ms at 128^3, profiles/r03_notes.md),
   // whole items 6000 (profiles/r02_notes.md)
-  if (p.stagger < 0) p.stagger = MW > 1 ? 3000 : 6000;
+  p.stagger = MW > 1 ? 3000 : 6000;
   if constexpr (MW > 1) {
     SB_CHECK(p.nranks == 1, SB200_ERR_SUP, "persistent path: split items are a single-GPU configuration");
   } else if (p.nranks > 1) {
-    const size_t smem_slab_a = smem + (size_t)NWARPS * P * 8 * sizeof(double);  // + the pencil items' staging blocks
+    const size_t smem_slab = smem + (size_t)NWARPS * P * 8 * sizeof(double);  // + the pencil items' staging blocks
     if (!XF(p, 32)) {
-      int blocks = sms;
-      if (const char* mc = getenv("SB200_MAX_CTAS")) blocks = atoi(mc) > 0 ? atoi(mc) : blocks;
+      const int blocks = (int)cap_ctas(sms);
       {
         // same shared-memory carve-out as the chain kernel that shares the SMs with it: an SM whose carve-out has to change
         // first drains, which delayed the chain kernel's CTAs behind the stage blocks (CTA starts spread over 12 us at 2 GPUs)
@@ -717,9 +721,7 @@ int run_cfg(PersistParams& p, cudaStream_t s) {
     }
     p.nlocal_items = (unsigned)(p.nlines / (8 * NT) * (p.d - 1 - p.first_axis));
     if (NT != 1) p.bulk = 0;
-    SB_TRY((launch_phase<P, NWARPS, NT, 1, false, true>(p, smem_slab_a, sms, s)));
-    if (!p.merged) SB_TRY((launch_phase<P, NWARPS, NT, 1, true, true>(p, smem, sms, s)));
-    return 0;
+    return launch_phase<P, NWARPS, NT, 1, false, true>(p, smem_slab, sms, s);
   }
   SB_TRY((launch_phase<P, NWARPS, NT, MW, false, false>(p, smem, sms, s)));
   SB_TRY((launch_phase<P, NWARPS, NT, MW, true, false>(p, smem, sms, s)));
@@ -738,17 +740,11 @@ bool elliptic_persist_supported(const EllipticCtx& e) {
 }
 
 int persist_run(int P, PersistParams& p, cudaStream_t s) {
-  static bool read_env = false;
-  static int stg = -1;
-  if (!read_env) {
-    const char* g = getenv("SB200_STAGGER");
-    stg = g ? atoi(g) : -1;
-    read_env = true;
-  }
-  p.stagger = stg;  // (< 0: the configuration's default, run_cfg)
 #ifdef SB200_ABLATE
   const char* xf = getenv("SB200_XFLAGS");
   p.xflags = xf ? atoi(xf) : 0;
+  const char* tl = getenv("SB200_TL_EPOCH");
+  p.tl_epoch = tl ? (unsigned long long)atoll(tl) : 0;
 #else
   p.xflags = 0;
 #endif

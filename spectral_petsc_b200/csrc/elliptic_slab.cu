@@ -1,15 +1,13 @@
 // Slab-partitioned MatMult_Elliptic (elliptic.C:297-339) over 2/4/8 GPUs: the grid is cut along its
 // outermost axis, one process per GPU.  Derivatives along the local axes never leave the GPU.  The
 // axis-0 chain  D_0 (eta D_0 w + eta' w g0)  runs on "pencils" (all P planes of 1/G of the lines):
-// the persistent chain kernel (elliptic_persist.cu) first pads its local input and pushes each plane's
-// lines into the owning rank's pencil with contiguous stores over NVLink (the forward all-to-all), runs
-// the local-axis items while those arrive, then the pencil items out of local memory, whose epilogue
-// stores the result rows straight into the plane owners' partial field (the backward all-to-all).  Ranks
-// order themselves with two epoch flags in peer memory (READY: my planes are in your pencil; DONE: all
-// my results are in your partial field), never through the host.  Two launches per application, as on
-// one GPU: phase A (push, local axes, pencil items), phase B (last axis; reads part[0] after DONE).
-#include <cstdlib>
-
+// a stage kernel (elliptic_persist.cu) pads the local input and pushes each plane's lines into the
+// owning rank's pencil with contiguous stores over NVLink (the forward all-to-all); the persistent chain
+// kernel, launched behind it, runs the local-axis items while those arrive, then the pencil items out of
+// local memory, whose epilogue stores the result rows straight into the plane owners' partial field (the
+// backward all-to-all), then the last-axis items, which read part[0] after DONE.  Ranks order themselves
+// with two epoch flags in peer memory (READY: my planes are in your pencil; DONE: all my results are in
+// your partial field), never through the host.
 #include "../../include/spectral_b200.h"
 #include "common.cuh"
 #include "deriv.h"
@@ -161,42 +159,17 @@ int elliptic_matmult_slab_fused(EllipticCtx& e, const double* U, double* V, cuda
   p.Rp = p.R0 / G;
   p.sf = sf;
   p.epoch = epoch;
-  {
-    // pencil results through TMA tensor stores (SB200_SLAB_BULK = 0 keeps the per-thread 16-byte peer stores of round 1)
-    static int bulk = -1;
-    if (bulk < 0) {
-      const char* c = getenv("SB200_SLAB_BULK");
-      bulk = c ? atoi(c) : 1;
+  // pencil results through TMA tensor stores (per-thread 16-byte peer stores when the descriptors cannot be encoded)
+  if (!e.tmaps_tried) {
+    e.tmaps_tried = true;
+    e.tmaps = new SlabMaps();
+    if (!encode_part0_maps(p.part0peer, G, p.R0, nloc, e.tmaps)) {
+      delete e.tmaps;
+      e.tmaps = nullptr;
     }
-    if (bulk && !e.tmaps_tried) {
-      e.tmaps_tried = true;
-      e.tmaps = new SlabMaps();
-      if (!encode_part0_maps(p.part0peer, G, p.R0, nloc, e.tmaps)) {
-        delete e.tmaps;
-        e.tmaps = nullptr;
-      }
-    }
-    p.maps = bulk ? e.tmaps : nullptr;
-    p.bulk = p.maps ? 1 : 0;
   }
-  {
-    // one launch for all axes (the last axis waits for the local items by a counter and for the peers by DONE) or the
-    // two PDL-chained phases of the single-GPU kernel: SB200_SLAB_MERGED = 0 / 1, default merged
-    static int merged = -1;
-    if (merged < 0) {
-      const char* c = getenv("SB200_SLAB_MERGED");
-      merged = c ? atoi(c) : 1;
-    }
-    p.merged = merged;
-  }
-  {
-    static long long tl = -1;
-    if (tl < 0) {
-      const char* c = getenv("SB200_TL_EPOCH");
-      tl = c ? atoll(c) : 0;
-    }
-    p.tl_epoch = (unsigned long long)tl;
-  }
+  p.maps = e.tmaps;
+  p.bulk = p.maps ? 1 : 0;
   p.trace = nullptr;
   return persist_run(P, p, s);
 }

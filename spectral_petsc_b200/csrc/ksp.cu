@@ -6,7 +6,6 @@
 #include "ksp.h"
 
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 
 #include "../../include/spectral_b200.h"
@@ -17,7 +16,6 @@ namespace sb200 {
 
 namespace {
 
-constexpr int CHMAX = 32;    // vectors per dot-product pass: template parameter CH in {8, 16, 32}; 8 is the default (measured), SB200_KSP_MDOT_CH raises it
 constexpr int TPB = 256;
 
 // The vector kernels of an Arnoldi step follow each other on one stream, each a few tens of microseconds long: launched as programmatic
@@ -346,8 +344,7 @@ int KspCtx::init(long long n_, int restart_, int rank, int nranks) {
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  int per_sm = 8;
-  if (const char* c = getenv("SB200_KSP_BLOCKS_PER_SM")) per_sm = atoi(c) > 0 ? atoi(c) : 8;  // tuning hook (8 measured best, profiles/r02_notes.md)
+  const int per_sm = 8;  // measured best (profiles/r02_notes.md)
   nblocks = (int)std::min<long long>((n + TPB - 1) / TPB > 0 ? (n + TPB - 1) / TPB : 1, (long long)sms * per_sm);
   SB_CUDA(cudaMalloc((void**)&partial, (size_t)nblocks * 64 * sizeof(double)));
   SB_CUDA(cudaMalloc((void**)&counters, 64 * sizeof(unsigned)));
@@ -375,15 +372,6 @@ KspCtx::~KspCtx() {
   arena.destroy();
 }
 
-static int maxpy_desc() {
-  static int d = -1;
-  if (d < 0) {
-    const char* c = getenv("SB200_KSP_DESC");  // tuning hook: MAXPY walks the vectors downwards (L2 reuse after the multi-dot)
-    d = c ? atoi(c) : 1;
-  }
-  return d;
-}
-
 int KspCtx::allreduce(double* vals, int k, cudaStream_t s) {
   if (arena.nranks == 1) return 0;
   SB_CHECK(arena.attached(), SB200_ERR_USER, "KSP on a slab partition: peers are not attached");
@@ -404,18 +392,8 @@ int KspCtx::allreduce(double* vals, int k, cudaStream_t s) {
 
 int KspCtx::dots(const double* x, const double* Y, long long ldy, int nv, double* out, cudaStream_t s) {
   const int vec2 = (reinterpret_cast<uintptr_t>(x) % 16 == 0 && reinterpret_cast<uintptr_t>(Y) % 16 == 0 && ldy % 2 == 0) ? 1 : 0;
-  static int chcap = -1;
-  if (chcap < 0) {
-    const char* c = getenv("SB200_KSP_MDOT_CH");  // tuning hook: largest group (8, 16 or 32 vectors per pass)
-    chcap = c ? atoi(c) : 8;  // measured on B200 (profiles/r02_notes.md): 8 vectors per pass beat 16 and 32 (registers, concurrent DRAM streams)
-  }
-  if (nv <= 8 || chcap <= 8) {
-    SB_CUDA(launch_pdl(mdot_kernel<8>, dim3(nblocks, (nv + 7) / 8), dim3(TPB), s, x, Y, ldy, nv, n, partial, counters, out, vec2));
-  } else if (nv <= 16 || chcap <= 16) {
-    mdot_kernel<16><<<dim3(nblocks, (nv + 15) / 16), TPB, 0, s>>>(x, Y, ldy, nv, n, partial, counters, out, vec2);
-  } else {
-    mdot_kernel<CHMAX><<<dim3(nblocks, (nv + CHMAX - 1) / CHMAX), TPB, 0, s>>>(x, Y, ldy, nv, n, partial, counters, out, vec2);
-  }
+  // 8 vectors per pass: measured on B200 (profiles/r02_notes.md) against 16 and 32 (registers, concurrent DRAM streams)
+  SB_CUDA(launch_pdl(mdot_kernel<8>, dim3(nblocks, (nv + 7) / 8), dim3(TPB), s, x, Y, ldy, nv, n, partial, counters, out, vec2));
   count_launch();
   SB_CUDA(cudaGetLastError());
   return allreduce(out, nv, s);
@@ -495,7 +473,7 @@ int KspCtx::solve(const double* b, double* x, bool guess_nonzero, cudaStream_t s
       ha.rnorm_dev = sp.scr + 3;
       ha.rnorm_host = d_rnorm + (kq % NRING);
       SB_CUDA(launch_pdl(maxpy_kernel, dim3(g1), dim3(TPB), s, w, (const double*)V, ld, kq + 1, (const double*)sp.hcol, -1.0, n, partial, counters + 32,
-                         sp.hcol + (kq + 1), 1, ha, maxpy_desc()));
+                         sp.hcol + (kq + 1), 1, ha, 1));  // desc = 1: L2 reuse after the multi-dot
       count_launch();
       if (!ha.on) {
         SB_TRY(allreduce(sp.hcol + (kq + 1), 1, s));

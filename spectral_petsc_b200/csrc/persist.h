@@ -44,9 +44,8 @@ struct PersistParams {
   unsigned long long epoch;             // READY / DONE flag value of this application
   int bulk;                             // slab: pencil results leave through TMA tensor stores (maps != nullptr) instead of per-thread stores
   const SlabMaps* maps;                 // host pointer (copied into the kernel's __grid_constant__ parameter at launch)
-  int merged;                           // slab: the last-axis items run in the same launch as phase A (no phase B launch)
-  unsigned nlocal_items;                // merged: local (non-pencil, non-last-axis) items whose partials the last axis reads
-  unsigned long long tl_epoch;          // debug timeline: the application to stamp (SB200_TL_EPOCH)
+  unsigned nlocal_items;                // slab: local (non-pencil, non-last-axis) items whose partials the last axis reads
+  unsigned long long tl_epoch;          // debug timeline (diagnostic builds): the application to stamp (SB200_TL_EPOCH)
   int stagger;       // start delay per warp group, in clocks
   int xflags;        // experiment switches (0 in production): 1 = no flux loads, 2 = no epilogue traffic
   long long* trace;  // optional (SB200_TRACE builds): per-item phase time stamps
@@ -59,8 +58,8 @@ struct alignas(64) SlabMaps {
   CUtensorMap m[SB200_MAX_RANKS];
 };
 
-// Runs phase A (axes first_axis..d-2; in slab mode also the axis-0 pencil items) and phase B (last
-// axis) for extent P in {32, 64, 128}.
+// Single GPU: runs phase A (axes 0..d-2) and phase B (last axis).  Slab mode: one launch runs the local axes, the
+// axis-0 pencil items and the last axis, extent P in {32, 64, 128}.
 int persist_run(int P, PersistParams& p, cudaStream_t s);
 
 }  // namespace sb200

@@ -6,8 +6,6 @@
 // (G-1)/G of the WHOLE field per rank for the operand-pull scheme (deriv_generic.cu slab mode), which this replaces
 // whenever the column count divides by the number of ranks.  The "field" is the scalar view (P planes x R columns,
 // element stride / offset for AoS components) that DerivParams describes.
-#include <cstdlib>
-
 #include "../../include/spectral_b200.h"
 #include "common.cuh"
 #include "deriv.h"
@@ -80,9 +78,8 @@ bool slab_deriv0_pencil_supported(const SymmArena& a, const DerivParams& p) {
 }
 
 // p: the slab-local description (x, y local arena arrays of this rank; O == 1; P = global extent; R columns).
-// Xp, Yp: arena arrays of at least P * R / nranks doubles.  Split in two so that the caller can put independent local
-// work between the operand push and the point where the peers' planes are needed.
-int slab_deriv0_pencil_begin(SymmArena& a, const DerivParams& p, int nloc, int i0, double* Xp, cudaStream_t s) {
+// Xp, Yp: arena arrays of at least P * R / nranks doubles.
+int slab_deriv0_pencil(SymmArena& a, const DerivParams& p, int nloc, int i0, double* Xp, double* Yp, cudaStream_t s) {
   SB_CHECK(a.attached(), SB200_ERR_USER, "slab partition: peers are not attached (exchange the IPC handles first)");
   const int G = a.nranks;
   const long long R = p.R, Rp = R / G;
@@ -91,22 +88,6 @@ int slab_deriv0_pencil_begin(SymmArena& a, const DerivParams& p, int nloc, int i
   push_to_pencils_kernel<<<blocks_for((long long)nloc * R), 256, 0, s>>>(p.x, p.xs, p.xoff, px, nloc, i0, R, Rp);
   count_launch();
   SB_CUDA(cudaGetLastError());
-  return 0;
-}
-
-SlabPush slab_make_push(const SymmArena& a, double* Xp, int i0, long long R) {
-  SlabPush sp;
-  for (int q = 0; q < SB200_MAX_RANKS; q++) sp.dst[q] = q < a.nranks ? a.on(q, Xp) : nullptr;
-  sp.on = 1;
-  sp.i0 = i0;
-  sp.R = R;
-  sp.Rp = R / a.nranks;
-  return sp;
-}
-
-int slab_deriv0_pencil_finish(SymmArena& a, const DerivParams& p, int nloc, double* Xp, double* Yp, cudaStream_t s) {
-  const int G = a.nranks;
-  const long long R = p.R, Rp = R / G;
   PushPtrs py;
   for (int q = 0; q < SB200_MAX_RANKS; q++) py.dst[q] = q < G ? a.on(q, p.y) : nullptr;
   SB_TRY(a.barrier(s));
@@ -120,13 +101,8 @@ int slab_deriv0_pencil_finish(SymmArena& a, const DerivParams& p, int nloc, doub
   lp.xoff = lp.yoff = 0;
   lp.npeer = 0;
   // unit-stride result in an aligned even column range: the derivative's epilogue stores the rows straight into the plane owners'
-  // fields over NVLink (no pencil result buffer, no second push kernel)
-  static int peer_epi = -1;
-  if (peer_epi < 0) {
-    const char* c = getenv("SB200_SLAB_PEER_EPILOGUE");
-    peer_epi = c ? atoi(c) : 1;
-  }
-  if (peer_epi && p.ys == 1 && p.yoff == 0 && p.sync && Rp % 8 == 0 && R % 2 == 0 && deriv_eo_supported(lp) &&
+  // fields over NVLink (no pencil result buffer, no second push kernel); otherwise the pencil result goes through push_to_slabs_kernel
+  if (p.ys == 1 && p.yoff == 0 && p.sync && Rp % 8 == 0 && R % 2 == 0 && deriv_eo_supported(lp) &&
       reinterpret_cast<uintptr_t>(Xp) % 16 == 0 && reinterpret_cast<uintptr_t>(p.y) % 16 == 0) {
     lp.y = nullptr;
     lp.peer_on = 1;
@@ -143,11 +119,6 @@ int slab_deriv0_pencil_finish(SymmArena& a, const DerivParams& p, int nloc, doub
   count_launch();
   SB_CUDA(cudaGetLastError());
   return a.barrier(s);
-}
-
-int slab_deriv0_pencil(SymmArena& a, const DerivParams& p, int nloc, int i0, double* Xp, double* Yp, cudaStream_t s) {
-  SB_TRY(slab_deriv0_pencil_begin(a, p, nloc, i0, Xp, s));
-  return slab_deriv0_pencil_finish(a, p, nloc, Xp, Yp, s);
 }
 
 }  // namespace sb200

@@ -10,7 +10,6 @@
 #include <algorithm>
 #include <cfloat>
 #include <cmath>
-#include <cstdlib>
 #include <vector>
 
 #include "../../include/spectral_b200.h"
@@ -58,7 +57,7 @@ __device__ __forceinline__ NodeInfo decode_node(const GridDesc& gd, long long id
 // Four nodes per thread and pass, all their loads issued before the first store (the kernel is latency bound otherwise).
 template <int NC>
 __global__ void pad_nodes_kernel(GridDesc gd, const double* __restrict__ src, int sstride, int soff,
-                                 const double* __restrict__ dir, double* __restrict__ local, SlabPush push) {
+                                 const double* __restrict__ dir, double* __restrict__ local) {
   constexpr int U = 4;
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long idx0 = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx0 < gd.m; idx0 += U * stride) {
@@ -79,10 +78,7 @@ __global__ void pad_nodes_kernel(GridDesc gd, const double* __restrict__ src, in
       const long long idx = idx0 + u * stride;
       if (idx >= gd.m) continue;
 #pragma unroll
-      for (int k = 0; k < NC; k++) {
-        local[idx * NC + k] = v[u][k];
-        if (push.on) push.store(idx * NC + k, v[u][k]);  // slab: the axis-0 derivative's operand goes to the owners' pencils right here
-      }
+      for (int k = 0; k < NC; k++) local[idx * NC + k] = v[u][k];
     }
   }
 }
@@ -177,7 +173,7 @@ struct DivDst {
 
 template <int D, bool FOLD = false>
 __global__ void vv_flux_kernel(long long m, const double* __restrict__ eta, const double* __restrict__ deta, VPtrs<D> p,
-                               const double* __restrict__ pl, GridDesc gd, DivDst dv, SlabPush push) {
+                               const double* __restrict__ pl, GridDesc gd, DivDst dv) {
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += stride) {
     double g[D][D], st[D][D], S0[D][D];
@@ -215,7 +211,6 @@ __global__ void vv_flux_kernel(long long m, const double* __restrict__ eta, cons
         double val = __dadd_rn(s, __dmul_rn(__dmul_rn(de, S0[j][k]), z));
         if (FOLD && j == k) val = __dadd_rn(val, -pli);
         p.v[j][i * D + k] = val;
-        if (j == 0 && push.on) push.store(i * D + k, val);  // slab: V_0, the operand of the axis-0 divergence term, straight to the pencils
       }
   }
 }
@@ -249,7 +244,7 @@ __device__ __forceinline__ double atomicMaxD(double* addr, double v) {
 // stokes.C:708-725 + rheology (stokes.C:1920-1944): s = sym(grad v), gamma = 1/2 s:s, eta/deta, V = eta*s, strain = s
 template <int D, bool FOLD = false>
 __global__ void rheology_kernel(long long m, Rheo r, double* __restrict__ eta, double* __restrict__ deta, VPtrs<D> p,
-                                double* __restrict__ minmax, const double* __restrict__ pl, GridDesc gd, DivDst dv, SlabPush push) {
+                                double* __restrict__ minmax, const double* __restrict__ pl, GridDesc gd, DivDst dv) {
   // p.s[j] (const view) and the written strain are the same arrays: strain is read raw and overwritten
   const long long stride = (long long)gridDim.x * blockDim.x;
   double lmin = DBL_MAX, lmax = -DBL_MAX;
@@ -301,7 +296,6 @@ __global__ void rheology_kernel(long long m, Rheo r, double* __restrict__ eta, d
         double val = __dmul_rn(e, s[j][k]);
         if (FOLD && j == k) val = __dadd_rn(val, -pl[i]);  // opt-in: V = eta*eps - p I, see vv_flux_kernel
         p.v[j][i * D + k] = val;
-        if (j == 0 && push.on) push.store(i * D + k, val);
         sw[j][i * D + k] = s[j][k];
       }
   }
@@ -559,17 +553,12 @@ int StokesCtx::init(int d, const int* dim, int rank, int nranks) {
   SB_CUDA(cudaMalloc((void**)&vG1, std::max<size_t>(8, (size_t)gv * sizeof(double))));
   SB_CUDA(cudaMalloc((void**)&minmax, 2 * sizeof(double)));
   SB_CUDA(cudaMalloc((void**)&sync, 64));
-  {
-    // side stream: on a slab partition the local-axis derivative batch runs there beside the axis-0 pencil chain; on one GPU the pressure
-    // pad + boundary extrapolation (small latency-bound kernels) run there beside the velocity pad and the gradient batch
-    const char* c = getenv("SB200_STOKES_SIDE_STREAM");  // 0: everything on the caller's stream (round 1's order)
-    if (!c || atoi(c)) {
-      SB_CUDA(cudaStreamCreateWithFlags(&aux_stream, cudaStreamNonBlocking));
-      SB_CUDA(cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
-      SB_CUDA(cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming));
-      SB_CUDA(cudaEventCreateWithFlags(&ev_pjoin, cudaEventDisableTiming));
-    }
-  }
+  // side stream: on a slab partition the local-axis derivative batch runs there beside the axis-0 pencil chain; on one GPU the pressure
+  // pad + boundary extrapolation (small latency-bound kernels) run there beside the velocity pad and the gradient batch
+  SB_CUDA(cudaStreamCreateWithFlags(&aux_stream, cudaStreamNonBlocking));
+  SB_CUDA(cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
+  SB_CUDA(cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming));
+  SB_CUDA(cudaEventCreateWithFlags(&ev_pjoin, cudaEventDisableTiming));
   SB_CUDA(cudaMemset(sync, 0, 64));
   for (int k = 0; k < d; k++) {
     Dax[k] = nullptr;
@@ -693,13 +682,7 @@ int StokesCtx::deriv_p(int axis, const double* x, int xs, int xoff, double* y, i
 }
 
 bool StokesCtx::batchable() const {
-  static int use = -1;
-  if (use < 0) {
-    const char* c = getenv("SB200_NO_EO");
-    const char* b = getenv("SB200_NO_BATCH");
-    use = ((c && atoi(c)) || (b && atoi(b))) ? 0 : 1;
-  }
-  if (!use || gd.d > SB200_EO_MAX_JOBS) return false;
+  if (gd.d > SB200_EO_MAX_JOBS) return false;
   if (arena.nranks > 1 && gd.stride[0] % arena.nranks != 0) return false;  // the axis-0 pencils need R0 % G == 0
   for (int k = 1; k < gd.d; k++)
     if (Dax[k] != Dax[0]) return false;
@@ -710,33 +693,12 @@ bool StokesCtx::batchable() const {
 // Single GPU, every axis within the even-odd kernel's reach (P <= SB200_EO_MAX_P): the scatters and AXPY chains around the
 // derivatives run inside the derivative launches (fused pad loader, fused crop-sum epilogue; deriv.h), whatever the extents.
 bool StokesCtx::fusable() const {
-  static int use = -1;
-  if (use < 0) {
-    const char* c = getenv("SB200_NO_EO");
-    const char* b = getenv("SB200_NO_BATCH");
-    const char* f = getenv("SB200_NO_FUSE");
-    use = ((c && atoi(c)) || (b && atoi(b)) || (f && atoi(f))) ? 0 : 1;
-  }
-  if (!use || arena.nranks > 1) return false;
+  if (arena.nranks > 1) return false;
   for (int k = 0; k < gd.d; k++) {
     DerivParams p = job_p(k, workP[0], 1, 0, workP[1], 1, 0, nullptr, DERIV_STORE);
     if (!deriv_eo_supported(p)) return false;
   }
   return true;
-}
-
-// Slab partition with the pencil path available for the velocity view: the producer of `field` (m*d doubles, unit stride) pushes it.
-SlabPush StokesCtx::push_for(const double* field) const {
-  static int fuse = -1;
-  if (fuse < 0) {
-    const char* c = getenv("SB200_SLAB_PRODUCER_PUSH");
-    fuse = c ? atoi(c) : 0;  // measured SLOWER at 2 GPUs (the producers then wait on NVLink: pad 13 + push 23 us -> 71 us fused), off by default
-  }
-  SlabPush none;
-  if (!fuse || arena.nranks == 1 || !arena.attached() || !batchable()) return none;
-  DerivParams p = job_v(0, field, workV[1], nullptr, DERIV_STORE);
-  if (!slab_deriv0_pencil_supported(arena, p)) return none;
-  return slab_make_push(arena, Xp, gd.i0, p.R);
 }
 
 EoLineMap StokesCtx::line_map(int axis, int nc) const {
@@ -757,7 +719,6 @@ EoLineMap StokesCtx::line_map(int axis, int nc) const {
 int StokesCtx::run_jobs(DerivParams* jobs, int d, cudaStream_t s) {
   if (arena.nranks == 1) return deriv_eo_jobs(jobs, d, sync, s);
   if (!slab_deriv0_pencil_supported(arena, jobs[0])) {
-    prefilled = nullptr;
     SB_TRY(deriv_common(jobs[0], 0, s));
     if (d > 1) SB_TRY(deriv_eo_batch(jobs + 1, d - 1, sync, s));
     return 0;
@@ -765,21 +726,14 @@ int StokesCtx::run_jobs(DerivParams* jobs, int d, cudaStream_t s) {
   // The axis-0 chain (push the operand planes into the pencils, barrier, differentiate the pencil, push the rows back, barrier) runs on
   // the caller's stream; the local axes run CONCURRENTLY on the context's side stream (their own ticket counters): the two pushes and the
   // two cross-GPU barriers no longer sit in front of / behind 40 us of local work (profiles/r02_stokes_slab_profile_n2.txt).
-  if (d > 1 && aux_stream) {
+  if (d > 1) {
     SB_CUDA(cudaEventRecord(ev_fork, s));
     SB_CUDA(cudaStreamWaitEvent(aux_stream, ev_fork, 0));
     SB_TRY(deriv_eo_batch(jobs + 1, d - 1, sync + 4, aux_stream));
     SB_CUDA(cudaEventRecord(ev_join, aux_stream));
   }
-  if (prefilled && prefilled == jobs[0].x && jobs[0].xs == 1 && jobs[0].xoff == 0) {
-    // the kernel that wrote the operand already stored it into the owners' pencils: nothing to push
-  } else {
-    SB_TRY(slab_deriv0_pencil_begin(arena, jobs[0], gd.dim[0], gd.i0, Xp, s));
-  }
-  prefilled = nullptr;
-  if (d > 1 && !aux_stream) SB_TRY(deriv_eo_batch(jobs + 1, d - 1, sync, s));
-  SB_TRY(slab_deriv0_pencil_finish(arena, jobs[0], gd.dim[0], Xp, Yp, s));
-  if (d > 1 && aux_stream) SB_CUDA(cudaStreamWaitEvent(s, ev_join, 0));
+  SB_TRY(slab_deriv0_pencil(arena, jobs[0], gd.dim[0], gd.i0, Xp, Yp, s));
+  if (d > 1) SB_CUDA(cudaStreamWaitEvent(s, ev_join, 0));
   return 0;
 }
 
@@ -809,20 +763,16 @@ int StokesCtx::crop_trace(double* const* grads, double* dst, int dstride, int do
   return 0;
 }
 
-int StokesCtx::pad_vel(const double* src, int sstride, int soff, bool with_dirichlet, double* local, cudaStream_t s, bool feeds_gradient) {
-  // (only the caller whose NEXT step is the velocity-view gradient of `local` may ask for the push: a push nobody consumes would race
-  // with the real pushes of the other ranks into the same pencils)
-  const SlabPush push = feeds_gradient ? push_for(local) : SlabPush();
-  if (gd.d == 2) pad_nodes_kernel<2><<<grid_for(gd.m), 256, 0, s>>>(gd, src, sstride, soff, with_dirichlet ? dirichlet : nullptr, local, push);
-  else pad_nodes_kernel<3><<<grid_for(gd.m), 256, 0, s>>>(gd, src, sstride, soff, with_dirichlet ? dirichlet : nullptr, local, push);
-  if (push.on) prefilled = local;
+int StokesCtx::pad_vel(const double* src, int sstride, int soff, bool with_dirichlet, double* local, cudaStream_t s) {
+  if (gd.d == 2) pad_nodes_kernel<2><<<grid_for(gd.m), 256, 0, s>>>(gd, src, sstride, soff, with_dirichlet ? dirichlet : nullptr, local);
+  else pad_nodes_kernel<3><<<grid_for(gd.m), 256, 0, s>>>(gd, src, sstride, soff, with_dirichlet ? dirichlet : nullptr, local);
   count_launch();
   SB_CUDA(cudaGetLastError());
   return 0;
 }
 
 int StokesCtx::pad_pres(const double* src, int sstride, int soff, double* local, cudaStream_t s) {
-  pad_nodes_kernel<1><<<grid_for(gd.m), 256, 0, s>>>(gd, src, sstride, soff, nullptr, local, SlabPush());
+  pad_nodes_kernel<1><<<grid_for(gd.m), 256, 0, s>>>(gd, src, sstride, soff, nullptr, local);
   count_launch();
   SB_CUDA(cudaGetLastError());
   return 0;
@@ -892,7 +842,7 @@ int StokesCtx::matmult_vv_into(const double* x, int xstride, int xoff, double* d
     }
     SB_TRY(run_jobs(jobs, d, s));
   } else {
-  SB_TRY(pad_vel(x, xstride, xoff, false, xL, s, true));                                       // :635-637
+  SB_TRY(pad_vel(x, xstride, xoff, false, xL, s));                                             // :635-637
   if (batchable()) {
     DerivParams jobs[3];
     for (int i = 0; i < d; i++) jobs[i] = job_v(i, xL, workV[2 + i], nullptr, DERIV_STORE);
@@ -907,19 +857,17 @@ int StokesCtx::matmult_vv_into(const double* x, int xstride, int xoff, double* d
   // knows the slab view, so this holds on a partition too)
   DivDst dv{nullptr, 0, 0};
   if (div_dst) dv = DivDst{div_dst, div_stride, div_off};
-  const SlabPush push = push_for(workV[2]);  // slab: the flux kernel fills the pencils of the tail's axis-0 term itself
-  if (push.on) prefilled = workV[2];
   SB_TRY(join_pressure(s));  // the folded pressure prepared on the side stream
   if (d == 2) {
     VPtrs<2> p;
     for (int j = 0; j < 2; j++) { p.v[j] = workV[2 + j]; p.s[j] = strain[j]; }
-    if (p_local) vv_flux_kernel<2, true><<<grid_for(gd.m), 256, 0, s>>>(gd.m, eta, deta, p, p_local, gd, dv, push);
-    else vv_flux_kernel<2><<<grid_for(gd.m), 256, 0, s>>>(gd.m, eta, deta, p, nullptr, gd, dv, push);
+    if (p_local) vv_flux_kernel<2, true><<<grid_for(gd.m), 256, 0, s>>>(gd.m, eta, deta, p, p_local, gd, dv);
+    else vv_flux_kernel<2><<<grid_for(gd.m), 256, 0, s>>>(gd.m, eta, deta, p, nullptr, gd, dv);
   } else {
     VPtrs<3> p;
     for (int j = 0; j < 3; j++) { p.v[j] = workV[2 + j]; p.s[j] = strain[j]; }
-    if (p_local) vv_flux_kernel<3, true><<<grid_for(gd.m), 256, 0, s>>>(gd.m, eta, deta, p, p_local, gd, dv, push);
-    else vv_flux_kernel<3><<<grid_for(gd.m), 256, 0, s>>>(gd.m, eta, deta, p, nullptr, gd, dv, push);
+    if (p_local) vv_flux_kernel<3, true><<<grid_for(gd.m), 256, 0, s>>>(gd.m, eta, deta, p, p_local, gd, dv);
+    else vv_flux_kernel<3><<<grid_for(gd.m), 256, 0, s>>>(gd.m, eta, deta, p, nullptr, gd, dv);
   }
   count_launch();
   SB_CUDA(cudaGetLastError());
@@ -991,7 +939,7 @@ int StokesCtx::pad_pres_reduced(const double* src, int sstride, int soff, double
 // extrapolation contains cross-rank barriers, which must stay in the one stream order every rank shares: serial there.
 int StokesCtx::fold_pressure_begin(const double* xG, cudaStream_t s) {
   const int d = gd.d;
-  if (arena.nranks == 1 && aux_stream) {
+  if (arena.nranks == 1) {
     SB_CUDA(cudaEventRecord(ev_fork, s));
     SB_CUDA(cudaStreamWaitEvent(aux_stream, ev_fork, 0));
     SB_TRY(pad_pres_reduced(xG, d + 1, d, workP[0], aux_stream));
@@ -1134,7 +1082,7 @@ int StokesCtx::function(const double* xG, double* yG, cudaStream_t s) {
     SB_TRY(fold_pressure_begin(xG, s));  // first (on one GPU on the side stream, beside the velocity pad and the gradient batch)
     pfold = workP[0];
   }
-  SB_TRY(pad_vel(xG, d + 1, 0, true, xL, s, true));                                           // :691-699
+  SB_TRY(pad_vel(xG, d + 1, 0, true, xL, s));                                                 // :691-699
   if (fusable() || batchable()) {
     DerivParams jobs[3];
     for (int i = 0; i < d; i++) jobs[i] = job_v(i, xL, strain[i], nullptr, DERIV_STORE);
@@ -1148,18 +1096,16 @@ int StokesCtx::function(const double* xG, double* yG, cudaStream_t s) {
   init_minmax_kernel<<<1, 1, 0, s>>>(minmax);
   count_launch();
   Rheo r{rheology, hardness, exponent, regularization, gamma0};
-  const SlabPush push = push_for(workV[2]);
-  if (push.on) prefilled = workV[2];
   if (d == 2) {
     VPtrs<2> p;
     for (int j = 0; j < 2; j++) { p.v[j] = workV[2 + j]; p.s[j] = strain[j]; }
-    if (pfold) rheology_kernel<2, true><<<grid_for(gd.m), 256, 0, s>>>(gd.m, r, eta, deta, p, minmax, pfold, gd, dv, push);
-    else rheology_kernel<2><<<grid_for(gd.m), 256, 0, s>>>(gd.m, r, eta, deta, p, minmax, nullptr, gd, dv, push);
+    if (pfold) rheology_kernel<2, true><<<grid_for(gd.m), 256, 0, s>>>(gd.m, r, eta, deta, p, minmax, pfold, gd, dv);
+    else rheology_kernel<2><<<grid_for(gd.m), 256, 0, s>>>(gd.m, r, eta, deta, p, minmax, nullptr, gd, dv);
   } else {
     VPtrs<3> p;
     for (int j = 0; j < 3; j++) { p.v[j] = workV[2 + j]; p.s[j] = strain[j]; }
-    if (pfold) rheology_kernel<3, true><<<grid_for(gd.m), 256, 0, s>>>(gd.m, r, eta, deta, p, minmax, pfold, gd, dv, push);
-    else rheology_kernel<3><<<grid_for(gd.m), 256, 0, s>>>(gd.m, r, eta, deta, p, minmax, nullptr, gd, dv, push);
+    if (pfold) rheology_kernel<3, true><<<grid_for(gd.m), 256, 0, s>>>(gd.m, r, eta, deta, p, minmax, pfold, gd, dv);
+    else rheology_kernel<3><<<grid_for(gd.m), 256, 0, s>>>(gd.m, r, eta, deta, p, minmax, nullptr, gd, dv);
   }
   count_launch();
   SB_CUDA(cudaGetLastError());

@@ -37,7 +37,8 @@ struct StokesCtx {
   unsigned* sync = nullptr;  // counters of the even-odd derivative kernel
   double* Xp = nullptr;   // pencil operand / result buffers of the axis-0 derivative (m*d doubles each)
   double* Yp = nullptr;
-  cudaStream_t aux_stream = nullptr;  // slab: the local-axis derivative batch runs here, beside the axis-0 pencil chain on the caller's stream
+  // slab: the local-axis derivative batch runs here, beside the axis-0 pencil chain on the caller's stream; single GPU: the folded pressure
+  cudaStream_t aux_stream = nullptr;
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_pjoin = nullptr;
   bool pressure_pending = false;  // the folded pressure is being prepared on the side stream (join_pressure before its consumer)
   int fold_pressure_begin(const double* xG, cudaStream_t s);
@@ -55,15 +56,13 @@ struct StokesCtx {
   // single GPU and every extent <= SB200_EO_MAX_P: pad / crop / AXPY chains run inside the derivative launches (deriv.h)
   bool fusable() const;
   EoLineMap line_map(int axis, int nc) const;
-  SlabPush push_for(const double* field) const;
-  const double* prefilled = nullptr;  // slab: the field whose producer kernel has just filled the axis-0 pencils (consumed by the next run_jobs)
   int run_jobs(DerivParams* jobs, int d, cudaStream_t s);
   int crop_sum(int nc, int nterms, double* const* terms, double sign, double* dst, int dstride, int doff, cudaStream_t s);
 
   int deriv_v(int axis, const double* x, double* y, const double* yin, int mode, cudaStream_t s);
   int deriv_p(int axis, const double* x, int xs, int xoff, double* y, int ys, int yoff, const double* yin, int mode,
               cudaStream_t s);
-  int pad_vel(const double* src, int sstride, int soff, bool with_dirichlet, double* local, cudaStream_t s, bool feeds_gradient = false);
+  int pad_vel(const double* src, int sstride, int soff, bool with_dirichlet, double* local, cudaStream_t s);
   int pad_pres(const double* src, int sstride, int soff, double* local, cudaStream_t s);
   int crop(int nc, const double* local, double* dst, int dstride, int doff, bool add, const double* sub, cudaStream_t s);
   int viscous_tail(double* dst, int dstride, int doff, cudaStream_t s);
